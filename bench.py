@@ -16,6 +16,10 @@ bit-identical to the reference module in fp32) on the host cores, on a bounded s
 `--workload prior` (not the default; BASELINE configs[3], SURVEY 8f-1) benches the latent-diffusion-prior path with
 the same contract: one "step" = one job of n=4096 samples per GPU = 50-step DDIM over the FiLM-MLP prior (T=1000, width
 1024, z_dim 32, beta_end 0.05) followed by the CondVAE decode to 64x64.
+
+`--dump-outputs DIR` writes the images the last timed step returned as DIR/images.npy (float32, [n_total, 1, 64, 64]).
+Weights, conditions and the Philox seed are fixed, so two builds run with the same arguments can be compared output for
+output.  Above DUMP_MAX_BYTES a fixed, seeded subset of the samples is written instead.
 """
 from __future__ import annotations
 
@@ -40,6 +44,7 @@ TC_CONV_NAMES = ["down1.net.3", "ds1", "down2.net.0", "down2.net.3", "ds2", "mid
 ATTN_SDPA_MMAC = 25.17                   # q k^T and p v of the 4 heads (SURVEY a4-L), not part of the conv figure
 SDE_STEPS, CFG, T_END = 300, 1.5, 0.005
 PEAKS_FALLBACK = {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0}
+DUMP_MAX_BYTES = 64_000_000             # --dump-outputs: bytes written in all, .npy headers included
 
 
 def shard_range(n_total: int, rank: int, world: int):
@@ -96,6 +101,24 @@ def report_comm(rank, world, local_rank, dev):
     print(f"[bench] NCCL {ver} comm rank {rank} nranks {world} cudaDev {local_rank} all_reduce(1) = {int(t.item())} "
           f"NCCL_DEBUG={os.environ.get('NCCL_DEBUG')} NCCL_DEBUG_FILE={os.environ.get('NCCL_DEBUG_FILE')}", file=sys.stderr, flush=True)
     assert int(t.item()) == world
+
+
+def dump_outputs(out_dir: str, outputs: dict) -> None:
+    """Write each tensor of `outputs` as <out_dir>/<name>.npy in float32.  The leading axis is the sample; when an array
+    would take more than its share of DUMP_MAX_BYTES, a fixed (seed 0), sorted subset of its samples is written."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    budget = DUMP_MAX_BYTES // len(outputs) - 4096          # room for the .npy header
+    for name, x in outputs.items():
+        x = x.detach().float()
+        n, row_bytes = x.shape[0], x[0].numel() * 4
+        if n * row_bytes > budget:
+            keep = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:budget // row_bytes].sort().values
+            x = x[keep.to(x.device)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), x.cpu().numpy())
+        print(f"[bench] {name}: {x.shape[0]} of {n} samples -> {os.path.join(out_dir, name + '.npy')}", file=sys.stderr,
+              flush=True)
 
 
 def load_peaks():
@@ -388,26 +411,28 @@ def run_gpu_prior(args):
         torch.cuda.synchronize()
 
     def timed(fn, k):
+        """(ms over k calls of fn, max over ranks; what the last call returned)"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
+        out = None
         for _ in range(k):
-            fn()
+            out = fn()
         e1.record()
         barrier()
-        return max_over_ranks(e0.elapsed_time(e1), dev)
+        return max_over_ranks(e0.elapsed_time(e1), dev), out
 
     for _ in range(args.warmup):
         job_device()
     l0 = prior.launch_count() + vae.launch_count()
     with ClockSampler(local_rank) as clk:
-        ms = timed(job_device, args.steps)
+        ms, images = timed(job_device, args.steps)
     launches = prior.launch_count() + vae.launch_count() - l0
     job_e2e()
-    ms_e2e = timed(job_e2e, args.steps)
+    ms_e2e, _ = timed(job_e2e, args.steps)
     # decode alone (device events on the current stream; the library orders its stream against it)
     z = torch.randn((n, 32), device=dev)
-    ms_dec = timed(lambda: vae.decode(z, y_cat, y_cont, z_mean=z_mean, z_std=z_std), 5) / 5
+    ms_dec = timed(lambda: vae.decode(z, y_cat, y_cont, z_mean=z_mean, z_std=z_std), 5)[0] / 5
     kms = (C.c_float * 4)()
     if rank == 0:
         _cabi.check(_cabi.lib().tcs_prior_profile(prior.engine_handle(sched), n, 20, kms))
@@ -415,6 +440,8 @@ def run_gpu_prior(args):
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         sps, cores, desc = cpu_prior_samples_per_sec(n=max(args.cpu_n, 512), steps=max(2, args.cpu_steps // 3))
         cpu = {"value": sps, "unit": "samples/s", "cores": cores, "kind": "port", "sample": desc}
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"images": images})
     if rank == 0:
         peaks = load_peaks()
         value = n_total * args.steps / (ms / 1e3)
@@ -566,27 +593,29 @@ def run_gpu(args):
         torch.cuda.synchronize()
 
     def timed(fn, k):
+        """(ms over k calls of fn, max over ranks; what the last call returned)"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
+        out = None
         for _ in range(k):
-            fn()
+            out = fn()
         e1.record()
         barrier()
-        return max_over_ranks(e0.elapsed_time(e1), dev)  # ms, max over ranks
+        return max_over_ranks(e0.elapsed_time(e1), dev), out
 
     for _ in range(args.warmup):
         job_device(args.warmup_sde_steps or SDE_STEPS)
     launches0 = model.launch_count()
     with ClockSampler(local_rank) as clk:
-        ms = timed(job_device, args.steps)
+        ms, images = timed(job_device, args.steps)
     launches = model.launch_count() - launches0
     if args.skip_e2e:
         ms_e2e = None
     else:
         if not args.warmup_sde_steps:   # (long strong-scaling jobs: the device jobs above already warmed everything)
             job_e2e()
-        ms_e2e = timed(job_e2e, args.steps)
+        ms_e2e, _ = timed(job_e2e, args.steps)
 
     kern = profile_kernels(model, sde, dev, n=args.profile_n) if rank == 0 else None
     extra = {}
@@ -596,6 +625,8 @@ def run_gpu(args):
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         sps, cores, kind, desc = cpu_reference_samples_per_sec(n=args.cpu_n, steps=args.cpu_steps)
         cpu = {"value": sps, "unit": "samples/s", "cores": cores, "kind": kind, "sample": desc}
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"images": images})
     if rank == 0:
         peaks = load_peaks()
         value = n_total * args.steps / (ms / 1e3)
@@ -818,7 +849,13 @@ def main():
     ap.add_argument("--cpu-steps", type=int, default=15)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-cuda-eager", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the images of the last timed step to DIR/images.npy (float32) for output comparisons")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the B200 implementation's outputs; it does not apply to --impl reference")
     if args.workload == "prior":
         return run_reference_prior(args) if args.impl == "reference" else run_gpu_prior(args)
     if args.impl == "reference":

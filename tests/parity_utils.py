@@ -47,6 +47,12 @@ def golden(name):
     return torch.load(os.path.join(GOLDEN, name), weights_only=False)
 
 
+def image_of(x0_hat):
+    """The reference's final map from the pre-clamp projection to the [0,1] image (bit-exact in fp32), so that the golden
+    files store x0_hat only."""
+    return ((x0_hat + 1.0) * 0.5).clamp(0.0, 1.0)
+
+
 def conv_reference(in0, in1, w, b, ksize, stride, round_bf16=False):
     """torch circular conv on NHWC fp32 inputs; returns NHWC fp32."""
     x = in0 if in1 is None else torch.cat([in0, in1], dim=-1)

@@ -81,12 +81,15 @@ def test_oracle_forward_matches_reference_golden(golden_dir):
 
 
 def test_oracle_sampler_matches_reference_golden(golden_dir):
-    g = _load(golden_dir, "samplers.pt")["sde_s3_cfg0.0"]
     sd = orc.default_init_state_dict(1)
-    tr = orc.sample(sd, orc.DEFAULT_CFG, orc.Schedule(0.1, 30.0), g["y_cat"], g["y_cont"], g["x_init"], "sde",
-                    g["steps"], g["cfg"], g["t_end"], g["noise"])
-    assert orc.rel_l2(tr.x0_hat, g["x0_hat"]) < 1e-5
-    assert len(tr.eps) == g["steps"] + 1
+    for key, g in _load(golden_dir, "samplers.pt").items():
+        tr = orc.sample(sd, orc.DEFAULT_CFG, orc.Schedule(0.1, 30.0), g["y_cat"], g["y_cont"], g["x_init"], g["sampler"],
+                        g["steps"], g["cfg"], g["t_end"], g["noise"])
+        assert orc.rel_l2(tr.x0_hat, g["x0_hat"]) < 1e-5, key
+        assert len(tr.eps) == len(g["eps"]) == (2 * g["steps"] + 1 if g["sampler"] == "ode" else g["steps"] + 1), key
+        k = g["eps"][0].shape[0]          # the stored traces hold the first k samples of the run
+        for e, e_ref in zip(tr.eps, g["eps"]):
+            assert orc.rel_l2(e[:k], e_ref) < 1e-5, key
 
 
 def test_oracle_zero_out_conv_is_linear_recurrence():
