@@ -137,12 +137,15 @@ def debug_conv_ups(in_lo, w, b):
     return out
 
 
-def debug_layer(m: CondUNetTiny, name, x, t, y_cat, y_cont, C_out, res):
+def debug_layer(m: CondUNetTiny, name, x, t, y_cat, y_cont, C_out, res, uncond=0):
+    """One layer's output of a network pass over x (NHWC fp32).  uncond=1 runs the CFG batch: 2n rows alternating
+    conditional / unconditional; its "eps" tap is the guided eps (guidance 1.5) of the n samples."""
     h = m.engine_handle()
     n = x.shape[0]
-    out = torch.full((n, res, res, C_out), float("nan"), device="cuda")
+    rows = n * (2 if uncond and name != "eps" else 1)
+    out = torch.full((rows, res, res, C_out), float("nan"), device="cuda")
     got = _cabi.lib().tcs_debug_layer(h, name.encode(), x.data_ptr(), t.data_ptr(), y_cat.data_ptr(), y_cont.data_ptr(),
-                                      n, 0, out.data_ptr(), out.numel(), None)
+                                      n, 1 if uncond else 0, out.data_ptr(), out.numel(), None)
     if got < 0:
         _cabi.check(int(got))
     torch.cuda.synchronize()

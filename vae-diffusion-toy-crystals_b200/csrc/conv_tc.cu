@@ -288,7 +288,21 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
   constexpr int SB = UPS ? 1 : SLAB_BUFS;
   constexpr uint32_t WARP_SLAB = SB * 32 * BLK * 2, SLAB_BYTES = EPI_WARPS * WARP_SLAB;
   float* bias_s = reinterpret_cast<float*>(smem_raw + (slab_base - ptx::smem_u32(smem_raw)) + SLAB_BYTES);
-  for (int i = threadIdx.x; i < p.ntot; i += blockDim.x) bias_s[i] = p.epi.bias[i];
+  for (int i = threadIdx.x; i < p.ntot; i += blockDim.x) {
+    float b = p.epi.bias[i];
+    if constexpr (EPI == EPI_GN_FUSED) {
+      // GroupNorm is shift invariant: the fused epilogue works on v + bias - K_g with K_g = the mean of the group's
+      // biases, so that a bias far from zero (trained weights: |mean| >> std of the group) costs neither fp16 stash bits
+      // (rounding 2^-11 |v + bias - K_g| instead of 2^-11 |v + bias|) nor the cancellation of E[v^2] - mean^2
+      constexpr int CPGN = N / 8;
+      const int g0 = i - i % CPGN;
+      float k = 0.f;
+#pragma unroll
+      for (int j = 0; j < CPGN; ++j) k += p.epi.bias[g0 + j];
+      b -= k * (1.0f / CPGN);
+    }
+    bias_s[i] = b;
+  }
   EpiFusedSmem* fs = reinterpret_cast<EpiFusedSmem*>(reinterpret_cast<uint8_t*>(bias_s) + (GEO == 1 ? bias_bytes_of(p.ntot) : EPI_BIAS_BYTES));
   if constexpr (EPI == EPI_GN_FUSED)
     for (int i = threadIdx.x; i < N; i += blockDim.x) { fs->gamma[i] = p.epi.gamma[i]; fs->beta[i] = p.epi.beta[i]; }
@@ -854,7 +868,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
         const int img = mt / G;
         float rv[2 * NGL];                     // (sum, sum of squares) per local group
         // Pass 1 reads the accumulator ONCE (32 columns at a time, next tcgen05.ld in flight): statistics in fp32, and the
-        // biased values are kept as fp16 (3 more mantissa bits than the bf16 output, satfinite): column blocks 0 and 1 in
+        // biased values (bias_s holds bias - K_g, see its load) are kept as fp16 (3 more mantissa bits than the bf16 output,
+        // satfinite): column blocks 0 and 1 in
         // this warp's two output staging blocks (same [32 px][64 B] swizzled rows as the bf16 output that replaces them in
         // place in pass 2; a lane only ever touches its own row), block 2 in 16 registers.  The TMEM set therefore goes
         // back to the MMA warps BEFORE the cross-CTA exchange (the accumulator hold time was the bound of the K = 864
@@ -1000,7 +1015,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
             const int g = c / CPGN;
             const float sc = gsm->rstd[g] * fs->gamma[c];
             gsm->scale[c] = 0.5f * sc;                                                  // h = y / 2 = v * scale + shift
-            gsm->shift[c] = 0.5f * (fs->beta[c] - gsm->mean[g] * sc);                   // the bias is inside the stashed values
+            gsm->shift[c] = 0.5f * (fs->beta[c] - gsm->mean[g] * sc);                   // mean and stash both exclude K_g
           }
         }
         epi_bar_sync(grp);
