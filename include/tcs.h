@@ -13,7 +13,7 @@
  *        <- CondUNetTiny.forward  (:243-266)  and  predict_eps_cfg (:402-423)
  *   tcs_sample
  *        <- sample_probability_flow_ode (:452-504), sample_reverse_sde_euler_maruyama (:507-569),
- *           VPSDE (:273-298)
+ *           VPSDE (:273-298); also DPM-Solver++(2M), which the reference does not have
  *   tcs_condition_grid
  *        <- save_sde_samples condition synthesis (:317-321)
  *
@@ -46,7 +46,10 @@ enum tcs_status {
 
 enum tcs_precision { TCS_FP32 = 0, TCS_BF16 = 1 };
 enum tcs_engine { TCS_ENGINE_AUTO = 0, TCS_ENGINE_SIMT = 1, TCS_ENGINE_TCGEN05 = 2 };
-enum tcs_sampler { TCS_SAMPLER_ODE = 0, TCS_SAMPLER_SDE = 1 };
+/* ODE: probability-flow ODE, Heun, quadratic time grid.  SDE: reverse VP-SDE, Euler-Maruyama.
+ * DPMPP_2M: DPM-Solver++(2M) (Lu et al. 2022, Algorithm 2) on the probability-flow ODE, times uniform in
+ *           log-SNR, one evaluation per step, deterministic (noise must be NULL).  Not in the reference. */
+enum tcs_sampler { TCS_SAMPLER_ODE = 0, TCS_SAMPLER_SDE = 1, TCS_SAMPLER_DPMPP_2M = 2 };
 
 typedef struct tcs_config {
   int32_t n_types;     /* CondUNetTiny(n_types, ...)                                  */
@@ -97,7 +100,7 @@ typedef struct tcs_sample_args {
   const int64_t* y_cat;         /* [n] */
   const float* y_cont;          /* [n,y_cont_dim] */
   const float* x_init;          /* [n,1,64,64] or NULL -> Philox N(0,1) */
-  const float* noise;           /* [steps,n,1,64,64] or NULL -> Philox N(0,1) (SDE only) */
+  const float* noise;           /* [steps,n,1,64,64] or NULL -> Philox N(0,1) (SDE only; NULL for DPMPP_2M) */
   uint64_t seed;                /* Philox key */
   uint64_t global_index_offset; /* index of sample 0 of this call in the whole job (sharding) */
   float* x_out;                 /* [n,1,64,64] images in [0,1] */
@@ -110,7 +113,7 @@ typedef struct tcs_sample_args {
 
 int tcs_sample(tcs_handle* h, const tcs_sample_args* args, void* stream);
 
-/* Number of network evaluations tcs_sample performs: ode (Heun) 2*steps+1, sde steps+1. */
+/* Number of network evaluations tcs_sample performs: ode (Heun) 2*steps+1, sde and dpm++2m steps+1. */
 int32_t tcs_nfe(int32_t sampler, int32_t steps);
 
 /* y_cat[i] = (offset+i) % n_types ; y_cont[i] = [0, theta_max*(offset+i)/(n_total-1), 0, ...]. */
@@ -130,9 +133,22 @@ int tcs_sde_update(tcs_handle* h, float* x, const float* eps, const float* noise
 int tcs_ode_update(tcs_handle* h, int32_t mode, float* x, float* x_pred, float* d0, const float* eps, int32_t n,
                    float t, float t_next, void* stream);
 
+/* The DPM-Solver++(2M) update kernel on its own (bit-exactness tests), in fp32 and in this order:
+ *   x0 = (x - sigma*eps)/alpha;  D = c1 == 0 ? x0 : c0*x0 + c1*x0_prev;  x <- a*x + m*D;  x0_prev <- x0
+ * (c1 == 0 is a first-order row: x0_prev is not read). */
+int tcs_dpm_update(tcs_handle* h, float* x, float* x0_prev, const float* eps, int32_t n, float alpha, float sigma, float a,
+                   float m, float c0, float c1, void* stream);
+
 /* Host-side schedule, exactly as the kernels use it (for tests): ts has steps+1 entries. */
 int tcs_time_grid_host(int32_t steps, double t_end, float* ts_host);
 int tcs_schedule_host(double beta_min, double beta_max, float t, float* beta, float* alpha, float* sigma);
+/* The DPM-Solver++(2M) schedule tcs_sample uses (steps >= 1): ts_host [steps+1] = times uniform in
+ * log-SNR lambda = log alpha - log sigma from t = 1 to t_end (endpoints exact), fp32; coef_host [steps][4] =
+ * (a, m, c0, c1) of every step, computed in double from the fp32 times and rounded once:
+ *   h = lambda(t_{i+1}) - lambda(t_i), a = sigma(t_{i+1})/sigma(t_i), m = alpha(t_{i+1})*(-expm1(-h)),
+ *   (c0, c1) = (1, 0) on step 0 and, when steps < 15, on the last step; else r = h_{i-1}/h_i, (1 + 1/(2r), -1/(2r)). */
+int tcs_dpm_schedule_host(int32_t steps, double t_end, double beta_min, double beta_max, float* ts_host,
+                          float* coef_host);
 
 /* Waits for the handle's enqueued work and returns its sticky status bits (then clears them):
  *   bit 0: a fused GroupNorm layer saw a pre-norm activation that may exceed the fp16 staging range; the eps / images of

@@ -94,15 +94,21 @@ int launch_gn_finalize(const float* partials, int slots, int B, int H, int W, in
 struct StepCoef {   // one row per time-grid index i (host-computed in fp32, see tcs_api.cu)
   float t, beta, sigma, alpha, dt, g_sqrt_dt, pad0, pad1;   // dt = ts[i+1]-ts[i]; g_sqrt_dt = sqrt(beta)*sqrt(|dt|)
 };
-enum StepMode : int { STEP_SDE = 0, STEP_ODE_PREDICT = 1, STEP_ODE_CORRECT = 2, STEP_FINAL = 3 };
+// DPM-Solver++(2M) row i (host-computed in double from the fp32 log-SNR grid, each rounded to fp32 once):
+// a = sigma_{i+1}/sigma_i, m = alpha_{i+1}*(-expm1(-h_i)), D = c0*x0 + c1*x0_prev; c1 == 0 marks a first-order row
+struct DpmCoef {
+  float a, m, c0, c1;
+};
+enum StepMode : int { STEP_SDE = 0, STEP_ODE_PREDICT = 1, STEP_ODE_CORRECT = 2, STEP_FINAL = 3, STEP_DPM2M = 4 };
 struct StepArgs {
   const StepCoef* coef;     // device table
+  const DpmCoef* dpm;       // DPM2M: device table beside `coef`, same row index
   const int* step_ptr;      // device step counter (row = *step_ptr + row_off)
   int row_off;
   int mode;
-  float* x;                 // [n,4096] state (read; written for SDE / ODE_CORRECT)
+  float* x;                 // [n,4096] state (read; written for SDE / ODE_CORRECT / DPM2M)
   float* x_pred;            // ODE: Euler predictor state
-  float* d0;                // ODE: first drift
+  float* d0;                // ODE: first drift; DPM2M: x0_prev (the data prediction of the previous step)
   const float* eps;         // [n,4096]
   const float* noise;       // injected z for all steps [steps,n_total,4096] or null -> Philox
   long long noise_step_stride;  // elements between consecutive steps in `noise`

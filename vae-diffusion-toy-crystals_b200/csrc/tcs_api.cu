@@ -1,5 +1,5 @@
 // tcs_api.cu — the C ABI (include/tcs.h): handle, weights, workspace, the score network pass,
-// the two samplers and their CUDA-graph replay.  No PyTorch types, no CPU fallback.
+// the three samplers (Heun ODE, Euler-Maruyama SDE, DPM-Solver++(2M)) and their CUDA-graph replay.  No PyTorch types, no CPU fallback.
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -52,6 +52,41 @@ struct Sched {
     return sqrtf(v < 1e-8f ? 1e-8f : v);
   }
 };
+
+// DPM-Solver++(2M) schedule: times uniform in log-SNR lambda = log alpha - log sigma from t = 1 to t_end (endpoints pinned),
+// stored as fp32 like time_grid_host; the coefficients of step i are computed in double from those fp32 times and rounded
+// to fp32 once.  Step 0 is first order, and so is the last step when steps < 15 (the "lower order final" rule).
+static void dpm_schedule_host(int steps, double t_end, double bmin, double bmax, float* ts, DpmCoef* k) {
+  const double d = bmax - bmin;
+  auto alpha = [&](double t) { return exp(-0.5 * (bmin * t + 0.5 * d * (t * t))); };
+  auto sigma = [&](double t) { const double a = alpha(t); return sqrt(fmax(1.0 - a * a, 1e-8)); };
+  auto lambda = [&](double t) { return log(alpha(t)) - log(sigma(t)); };
+  const double l_start = lambda(1.0), l_end = lambda(t_end);
+  ts[0] = 1.0f;
+  for (int i = 1; i < steps; ++i) {
+    const double l = l_start + (static_cast<double>(i) / steps) * (l_end - l_start);
+    const double ib = log1p(exp(-2.0 * l));   // int_0^t beta = -2 log alpha, and alpha^2 = 1 / (1 + exp(-2 lambda))
+    ts[i] = static_cast<float>(d > 0.0 ? (-bmin + sqrt(bmin * bmin + 2.0 * d * ib)) / d : ib / bmin);
+  }
+  if (steps >= 1) ts[steps] = static_cast<float>(t_end);
+  double h_prev = 0.0;
+  for (int i = 0; i < steps; ++i) {
+    const double t0 = ts[i], t1 = ts[i + 1];
+    const double h = lambda(t1) - lambda(t0);
+    DpmCoef c;
+    c.a = static_cast<float>(sigma(t1) / sigma(t0));
+    c.m = static_cast<float>(alpha(t1) * -expm1(-h));
+    if (i == 0 || (i == steps - 1 && steps < 15)) {
+      c.c0 = 1.0f; c.c1 = 0.0f;
+    } else {
+      const double r = h_prev / h;
+      c.c0 = static_cast<float>(1.0 + 1.0 / (2.0 * r));
+      c.c1 = static_cast<float>(-1.0 / (2.0 * r));
+    }
+    k[i] = c;
+    h_prev = h;
+  }
+}
 
 
 enum ConvId { C_D1B, C_DS1, C_D2A, C_D2B, C_DS2, C_MA, C_MB, C_QKV, C_PROJ, C_US2, C_U2A, C_U2B, C_US1, C_U1A, C_U1B, C_COUNT };
@@ -133,7 +168,7 @@ struct tcs_handle {
   bool tc_out = false, eps_kxn = true;
 
   // per-call state
-  DevBuf cvec, tvec, tvals, coef, x, xpred, d0, eps, step_ctr, ycat_tmp, ycont_tmp;
+  DevBuf cvec, tvec, tvals, coef, dpm_coef, x, xpred, d0, eps, step_ctr, ycat_tmp, ycont_tmp;
   DevBuf status;                          // device status word (bit 0: fp16 stash range exceeded in a fused GroupNorm layer)
   void* pinned = nullptr; size_t pinned_bytes = 0;
   cudaEvent_t ev_pinned = nullptr;
@@ -147,7 +182,7 @@ struct tcs_handle {
   int64_t graph_kernels = 0;
 
   tcs_handle() {
-    for (DevBuf* b : {&cvec, &tvec, &tvals, &coef, &x, &xpred, &d0, &eps, &step_ctr}) b->gen = &ws_gen;
+    for (DevBuf* b : {&cvec, &tvec, &tvals, &coef, &dpm_coef, &x, &xpred, &d0, &eps, &step_ctr}) b->gen = &ws_gen;
   }
 
   ~tcs_handle() {
@@ -843,6 +878,15 @@ int tcs_schedule_host(double bmin, double bmax, float t, float* beta, float* alp
   if (sigma) *sigma = s.sigma(t);
   return TCS_OK;
 }
+int tcs_dpm_schedule_host(int32_t steps, double t_end, double bmin, double bmax, float* ts, float* coef) {
+  if (steps < 1 || !ts || !coef) return fail(TCS_ERR_BAD_ARGUMENT, "tcs_dpm_schedule_host: steps >= 1, ts and coef required");
+  if (!(t_end > 0.0 && t_end < 1.0)) return fail(TCS_ERR_BAD_ARGUMENT, "tcs_dpm_schedule_host: t_end must be in (0,1)");
+  if (!(bmin > 0.0 && bmax >= bmin)) return fail(TCS_ERR_BAD_ARGUMENT, "tcs_dpm_schedule_host: need 0 < beta_min <= beta_max");
+  std::vector<DpmCoef> k(steps);
+  dpm_schedule_host(steps, t_end, bmin, bmax, ts, k.data());
+  memcpy(coef, k.data(), sizeof(DpmCoef) * steps);
+  return TCS_OK;
+}
 
 int tcs_create(tcs_handle** out, const tcs_config* cfg) {
   if (!out || !cfg) return fail(TCS_ERR_BAD_ARGUMENT, "tcs_create: null argument");
@@ -1182,39 +1226,79 @@ int tcs_ode_update(tcs_handle* h, int32_t mode, float* x, float* x_pred, float* 
   return leave(h, user);
 }
 
+int tcs_dpm_update(tcs_handle* h, float* x, float* x0_prev, const float* eps, int32_t n, float alpha, float sigma, float a,
+                   float m, float c0, float c1, void* stream) {
+  if (!h || !x || !x0_prev || !eps || n < 0) return fail(TCS_ERR_BAD_ARGUMENT, "tcs_dpm_update: bad argument");
+  if (n == 0) return TCS_OK;
+  TCS_CUDA(cudaSetDevice(h->cfg.device));
+  cudaStream_t user = static_cast<cudaStream_t>(stream);
+  TCS_CHECK(enter(h, user));
+  TCS_CHECK(h->coef.ensure(sizeof(StepCoef) * 8));
+  TCS_CHECK(h->dpm_coef.ensure(sizeof(DpmCoef) * 8));
+  TCS_CHECK(ensure_pinned(h, sizeof(StepCoef) * 8 + 64));
+  StepCoef* c = static_cast<StepCoef*>(h->pinned);
+  memset(c, 0, sizeof(StepCoef));
+  c->alpha = alpha; c->sigma = sigma;
+  DpmCoef* k = reinterpret_cast<DpmCoef*>(c + 1);
+  *k = DpmCoef{a, m, c0, c1};
+  TCS_CUDA(cudaMemcpyAsync(h->coef.p, c, sizeof(StepCoef), cudaMemcpyHostToDevice, h->stream));
+  TCS_CUDA(cudaMemcpyAsync(h->dpm_coef.p, k, sizeof(DpmCoef), cudaMemcpyHostToDevice, h->stream));
+  TCS_CUDA(cudaEventRecord(h->ev_pinned, h->stream));
+  StepArgs s{};
+  s.coef = h->coef.as<StepCoef>(); s.dpm = h->dpm_coef.as<DpmCoef>();
+  s.step_ptr = nullptr; s.row_off = 0;
+  s.mode = STEP_DPM2M; s.x = x; s.d0 = x0_prev; s.eps = eps; s.n = n;
+  ++h->launches;
+  TCS_CHECK(launch_step(s, h->stream));
+  return leave(h, user);
+}
+
 int tcs_sample(tcs_handle* h, const tcs_sample_args* args, void* stream) {
   TCS_CHECK(check_ready(h, "tcs_sample"));
   if (!args) return fail(TCS_ERR_BAD_ARGUMENT, "tcs_sample: null args");
   const tcs_sample_args& A = *args;
   if (!(A.t_end > 0.0 && A.t_end < 1.0))
     return fail(TCS_ERR_BAD_ARGUMENT, "t_end must be in (0,1), got " + std::to_string(A.t_end));
-  if (A.sampler != TCS_SAMPLER_ODE && A.sampler != TCS_SAMPLER_SDE)
-    return fail(TCS_ERR_BAD_ARGUMENT, "Unknown sampler. Use 'ode' or 'sde'.");
+  if (A.sampler != TCS_SAMPLER_ODE && A.sampler != TCS_SAMPLER_SDE && A.sampler != TCS_SAMPLER_DPMPP_2M)
+    return fail(TCS_ERR_BAD_ARGUMENT, "Unknown sampler. Use 'ode', 'sde' or 'dpm++2m'.");
+  if (A.sampler == TCS_SAMPLER_DPMPP_2M && A.noise)
+    return fail(TCS_ERR_BAD_ARGUMENT, "tcs_sample: the dpm++2m sampler is deterministic; noise must be NULL");
   if (A.n < 0 || A.steps < 0) return fail(TCS_ERR_BAD_ARGUMENT, "tcs_sample: n and steps must be >= 0");
   if (A.n == 0) return TCS_OK;
   if (!A.y_cat || !A.y_cont || !A.x_out) return fail(TCS_ERR_BAD_ARGUMENT, "tcs_sample: y_cat, y_cont and x_out are required");
   const int n = A.n, steps = A.steps;
   const int dup = A.guidance > 0.f ? 2 : 1;
   const bool ode = A.sampler == TCS_SAMPLER_ODE;
+  const bool dpm = A.sampler == TCS_SAMPLER_DPMPP_2M;
+  const Sched sc = A.beta_max > 0.0 ? Sched{A.beta_min, A.beta_max} : Sched{h->cfg.beta_min, h->cfg.beta_max};
+  if (dpm && !(sc.bmin > 0.0 && sc.bmax >= sc.bmin))
+    return fail(TCS_ERR_BAD_ARGUMENT, "tcs_sample: the dpm++2m sampler needs 0 < beta_min <= beta_max");
   cudaStream_t user = static_cast<cudaStream_t>(stream);
   TCS_CHECK(enter(h, user));
   cudaStream_t st = h->stream;
   const size_t img = static_cast<size_t>(n) * 4096 * 4;
   TCS_CHECK(h->x.ensure(img)); TCS_CHECK(h->eps.ensure(img));
   if (ode) { TCS_CHECK(h->xpred.ensure(img)); TCS_CHECK(h->d0.ensure(img)); }
+  if (dpm) { TCS_CHECK(h->d0.ensure(img)); TCS_CHECK(h->dpm_coef.ensure(sizeof(DpmCoef) * (steps + 1))); }   // d0 = x0_prev
   TCS_CHECK(h->cvec.ensure(static_cast<size_t>(n) * dup * 96 * 4));
   TCS_CHECK(h->tvec.ensure(static_cast<size_t>(steps + 1) * 96 * 4));
   TCS_CHECK(h->tvals.ensure(static_cast<size_t>(steps + 1) * 4));
   TCS_CHECK(h->coef.ensure(sizeof(StepCoef) * (steps + 2)));
 
   // ---- tables: time grid, schedule coefficients, embeddings --------------------------------------
-  const size_t pin_bytes = sizeof(StepCoef) * (steps + 2) + 4 * (steps + 1) + 64;
+  const size_t pin_bytes = sizeof(StepCoef) * (steps + 2) + (dpm ? sizeof(DpmCoef) * (steps + 1) : 0) + 4 * (steps + 1) + 64;
   TCS_CHECK(ensure_pinned(h, pin_bytes));
   StepCoef* hc = static_cast<StepCoef*>(h->pinned);
-  float* hts = reinterpret_cast<float*>(hc + steps + 2);
-  if (steps >= 1) time_grid_host(steps, A.t_end, hts);
-  else hts[0] = static_cast<float>(A.t_end) + static_cast<float>(1.0 - A.t_end);  // linspace(0,1,1) = [0]
-  const Sched sc = A.beta_max > 0.0 ? Sched{A.beta_min, A.beta_max} : Sched{h->cfg.beta_min, h->cfg.beta_max};
+  DpmCoef* hk = reinterpret_cast<DpmCoef*>(hc + steps + 2);
+  float* hts = dpm ? reinterpret_cast<float*>(hk + steps + 1) : reinterpret_cast<float*>(hc + steps + 2);
+  if (dpm) {
+    if (steps >= 1) dpm_schedule_host(steps, A.t_end, sc.bmin, sc.bmax, hts, hk);
+    else hts[0] = 1.0f;   // no step: the projection of x_T at t = 1, as for the other samplers
+  } else if (steps >= 1) {
+    time_grid_host(steps, A.t_end, hts);
+  } else {
+    hts[0] = static_cast<float>(A.t_end) + static_cast<float>(1.0 - A.t_end);  // linspace(0,1,1) = [0]
+  }
   for (int i = 0; i <= steps; ++i) {
     StepCoef c{};
     c.t = hts[i]; c.beta = sc.beta(c.t); c.sigma = sc.sigma(c.t); c.alpha = sc.alpha(c.t);
@@ -1223,6 +1307,7 @@ int tcs_sample(tcs_handle* h, const tcs_sample_args* args, void* stream) {
     hc[i] = c;
   }
   TCS_CUDA(cudaMemcpyAsync(h->coef.p, hc, sizeof(StepCoef) * (steps + 1), cudaMemcpyHostToDevice, st));
+  if (dpm && steps >= 1) TCS_CUDA(cudaMemcpyAsync(h->dpm_coef.p, hk, sizeof(DpmCoef) * steps, cudaMemcpyHostToDevice, st));
   TCS_CUDA(cudaMemcpyAsync(h->tvals.p, hts, 4 * (steps + 1), cudaMemcpyHostToDevice, st));
   TCS_CUDA(cudaEventRecord(h->ev_pinned, st));
   TCS_CUDA(cudaMemsetAsync(h->step_ctr.p, 0, 4, st));
@@ -1243,19 +1328,19 @@ int tcs_sample(tcs_handle* h, const tcs_sample_args* args, void* stream) {
 
   auto step_args = [&](int mode, int row_off) {
     StepArgs a{};
-    a.coef = h->coef.as<StepCoef>(); a.step_ptr = sp; a.row_off = row_off; a.mode = mode;
+    a.coef = h->coef.as<StepCoef>(); a.dpm = h->dpm_coef.as<DpmCoef>(); a.step_ptr = sp; a.row_off = row_off; a.mode = mode;
     a.x = x; a.x_pred = h->xpred.as<float>(); a.d0 = h->d0.as<float>(); a.eps = eps;
     a.noise = A.noise; a.noise_step_stride = static_cast<long long>(n) * 4096;
     a.seed = A.seed; a.gidx0 = A.global_index_offset; a.n = n;
     return a;
   };
   auto enqueue_step = [&]() -> int {
-    if (!ode) {
+    if (!ode) {   // SDE and DPM-Solver++(2M): one evaluation per step
       TCS_CHECK(trace_copy(h, A.trace_x, x, sp, 1, 0, n, st));
       TCS_CHECK(forward_all(h, x, cvec, tvec, 0, sp, 0, n, dup, A.guidance, eps, st));
       TCS_CHECK(trace_copy(h, A.trace_eps, eps, sp, 1, 0, n, st));
       ++h->launches;
-      TCS_CHECK(launch_step(step_args(STEP_SDE, 0), st));
+      TCS_CHECK(launch_step(step_args(dpm ? STEP_DPM2M : STEP_SDE, 0), st));
     } else {
       TCS_CHECK(trace_copy(h, A.trace_x, x, sp, 2, 0, n, st));
       TCS_CHECK(forward_all(h, x, cvec, tvec, 0, sp, 0, n, dup, A.guidance, eps, st));

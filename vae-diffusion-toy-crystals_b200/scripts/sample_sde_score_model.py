@@ -1,7 +1,8 @@
 #!/usr/bin/env python3
 """Same command line as the reference's scripts/sample_sde_score_model.py (:30-131): same flags,
 defaults, checkpoint layout ({"config","model",["ema"]}), default output name and final print.
-Additions: --precision {bf16,fp32} and --out-tensor (dump all n samples as a .pt tensor).
+Additions: --precision {bf16,fp32}, --out-tensor (dump all n samples as a .pt tensor) and --sampler dpm++2m
+(DPM-Solver++(2M): one network evaluation per step; 20 steps is the usual choice).
 
     python scripts/sample_sde_score_model.py --out-dir runs/sde --steps 300 --cfg 1.5 \
         --t-end 0.005 --sampler sde --use-ema 1
@@ -15,8 +16,7 @@ import torch
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."))
 from toycrystals_b200.models.sde_score_model import (  # noqa: E402
-    CondUNetTiny, VPSDE, condition_grid, sample_probability_flow_ode, sample_reverse_sde_euler_maruyama,
-    save_sde_samples)
+    _SAMPLERS, CondUNetTiny, VPSDE, condition_grid, save_sde_samples)
 
 
 def _infer_ckpt_path(out_dir: str, ckpt: str) -> str:
@@ -38,7 +38,7 @@ def main(argv=None) -> int:
     p.add_argument("--theta-max", type=float, default=math.pi / 3.0)
     p.add_argument("--n", type=int, default=36)
     p.add_argument("--use-ema", type=int, default=0, choices=[0, 1], help="If checkpoint has EMA weights, sample using them.")
-    p.add_argument("--sampler", type=str, default="ode", choices=["ode", "sde"])
+    p.add_argument("--sampler", type=str, default="ode", choices=list(_SAMPLERS))
     # fallback model / SDE config, used only when the checkpoint has no payload["config"]
     p.add_argument("--n-types", type=int, default=4)
     p.add_argument("--y-cont-dim", type=int, default=4)
@@ -84,7 +84,7 @@ def main(argv=None) -> int:
 
     if args.out_tensor:
         y_cat, y_cont = condition_grid(model, args.n, args.theta_max, device)
-        fn = sample_probability_flow_ode if args.sampler == "ode" else sample_reverse_sde_euler_maruyama
+        fn = _SAMPLERS[args.sampler]
         x = fn(model=model, sde=sde, y_cat=y_cat, y_cont=y_cont, img_shape=(args.n, 1, 64, 64), n_steps=args.steps,
                guidance_scale=args.cfg, t_end=args.t_end)
         torch.save(x.cpu(), args.out_tensor)

@@ -12,7 +12,7 @@ LIB_PATH = os.path.join(_HERE, "libtcs.so")
 TCS_OK, ERR_BAD_ARGUMENT, ERR_UNSUPPORTED, ERR_CUDA, ERR_STATE = 0, -1, -2, -3, -4
 FP32, BF16 = 0, 1
 ENGINE_AUTO, ENGINE_SIMT, ENGINE_TCGEN05 = 0, 1, 2
-SAMPLER_ODE, SAMPLER_SDE = 0, 1
+SAMPLER_ODE, SAMPLER_SDE, SAMPLER_DPMPP_2M = 0, 1, 2
 
 
 class TcsConfig(C.Structure):
@@ -65,7 +65,11 @@ SIGNATURES = {
                                  C.c_uint64, C.c_uint64, C.c_int32, C.c_void_p]),
     "tcs_ode_update": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
                                  C.c_float, C.c_float, C.c_void_p]),
+    "tcs_dpm_update": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32] + [C.c_float] * 6
+                       + [C.c_void_p]),
     "tcs_time_grid_host": (C.c_int, [C.c_int32, C.c_double, C.POINTER(C.c_float)]),
+    "tcs_dpm_schedule_host": (C.c_int, [C.c_int32, C.c_double, C.c_double, C.c_double, C.POINTER(C.c_float),
+                                        C.POINTER(C.c_float)]),
     "tcs_schedule_host": (C.c_int, [C.c_double, C.c_double, C.c_float, C.POINTER(C.c_float), C.POINTER(C.c_float),
                                     C.POINTER(C.c_float)]),
     "tcs_launch_count": (C.c_int64, [C.c_void_p]),

@@ -7,6 +7,7 @@ error behaviour — with every computation done by libtcs.so (hand-written sm_10
     predict_eps_cfg                    (:402-423)  -> tcs_score, CFG as ONE doubled batch
     sample_probability_flow_ode        (:452-504)  -> tcs_sample (Heun)
     sample_reverse_sde_euler_maruyama  (:507-569)  -> tcs_sample (Euler-Maruyama)
+    sample_dpmpp_2m                    (addition)  -> tcs_sample (DPM-Solver++(2M), one evaluation per step)
     save_sde_samples                   (:301-355)  condition grid + sampler + 6x6 PNG
 
 PyTorch is used for device memory, streams and the state-dict container only.  There is no CPU
@@ -434,6 +435,23 @@ def sample_reverse_sde_euler_maruyama(model: CondUNetTiny, sde: VPSDE, y_cat: to
                    return_trace=return_trace)
 
 
+@torch.no_grad()
+def sample_dpmpp_2m(model: CondUNetTiny, sde: VPSDE, y_cat: torch.Tensor, y_cont: torch.Tensor,
+                    img_shape: Tuple[int, int, int, int], n_steps: int = 20, guidance_scale: float = 0.0,
+                    t_end: float = 1e-3, *, x_init=None, seed=None, global_index_offset: int = 0,
+                    return_trace: bool = False):
+    """Deterministic sampler: DPM-Solver++(2M) (Lu et al. 2022, Algorithm 2) on the probability-flow ODE, times
+    uniform in log-SNR from t = 1 to t_end, first-order first step (and last step when n_steps < 15), one network
+    evaluation per step, final x0 projection; returns [B,1,64,64] in [0,1].  n_steps + 1 evaluations in all, against
+    2 n_steps + 1 for the Heun ODE sampler.  ``x_init`` / ``seed`` / ``global_index_offset`` / ``return_trace`` as for
+    the other samplers; the trace has the SDE sampler's layout."""
+    return _sample(model, sde, y_cat, y_cont, img_shape, n_steps, guidance_scale, t_end, _cabi.SAMPLER_DPMPP_2M,
+                   x_init=x_init, seed=seed, global_index_offset=global_index_offset, return_trace=return_trace)
+
+
+_SAMPLERS = {"ode": sample_probability_flow_ode, "sde": sample_reverse_sde_euler_maruyama, "dpm++2m": sample_dpmpp_2m}
+
+
 def condition_grid(model: CondUNetTiny, n: int, theta_max: float, device, offset: int = 0, n_total: Optional[int] = None):
     """y_cat[i] = i % n_types, y_cont[i] = [0, linspace(0, theta_max, n)[i], 0, ...] (reference :317-321),
     generated on the device by libtcs; (offset, n_total) select a shard of a larger grid."""
@@ -473,11 +491,11 @@ def save_sde_samples(model: CondUNetTiny, sde: VPSDE, out_path: str, device: tor
     CondUNetTiny or any module with the reference state dict (the training script's hook passes its own)."""
     model.eval()
     device = torch.device(device)
-    if sampler not in ("ode", "sde"):
-        raise ValueError(f"Unknown sampler='{sampler}'. Use 'ode' or 'sde'.")
+    if sampler not in _SAMPLERS:
+        raise ValueError(f"Unknown sampler='{sampler}'. Use 'ode', 'sde' or 'dpm++2m'.")
     model = adopt(model)
     y_cat, y_cont = condition_grid(model, n, theta_max, device)
-    fn = sample_probability_flow_ode if sampler == "ode" else sample_reverse_sde_euler_maruyama
+    fn = _SAMPLERS[sampler]
     x = fn(model=model, sde=sde, y_cat=y_cat, y_cont=y_cont, img_shape=(n, 1, 64, 64), n_steps=steps,
            guidance_scale=cfg, t_end=t_end)
     _write_grid_png(x, out_path, f"{sampler} | steps={steps} | cfg={cfg:.2f} | t_end={t_end:g}")
