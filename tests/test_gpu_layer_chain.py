@@ -240,10 +240,10 @@ def test_production_pass_layer_by_layer(scale, tval):
 
 
 # ---- B: the same chain under other grids: bit-identical outputs ---------------------------------------------------
-def _fresh_model(sd, chunk):
+def _fresh_model(sd, chunk, precision="bf16", engine="auto"):
     from toycrystals_b200.models.sde_score_model import CondUNetTiny
     pu = _pu()
-    m = CondUNetTiny(**pu.CFG, precision="bf16", chunk=chunk)
+    m = CondUNetTiny(**pu.CFG, precision=precision, engine=engine, chunk=chunk)
     m.load_state_dict(sd)
     return m.cuda().eval()
 

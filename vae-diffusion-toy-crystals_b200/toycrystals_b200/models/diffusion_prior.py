@@ -22,7 +22,7 @@ import torch
 import torch.nn as nn
 
 from .. import _cabi
-from .sde_score_model import _as_f32, _ptr, _stream_ptr, _write_grid_png
+from .sde_score_model import _as_f32, _ptr, _stream_ptr, _write_grid_png, params_checksum
 
 _PRECISIONS = {"fp32": _cabi.FP32, "bf16": _cabi.BF16}
 
@@ -70,7 +70,17 @@ class DiffusionPriorFiLM(nn.Module):
         self.use_graph = bool(use_graph)
         self._handle: Optional[C.c_void_p] = None
         self._handle_key = None
+        self._checksum = None
         self._sched_key = (1000, 1e-4, 0.05)
+
+    def refresh(self) -> "DiffusionPriorFiLM":
+        """Re-read the parameters on the next call if they changed behind autograd's back (``p.data.copy_(...)``, an EMA
+        update), which ``_version`` does not record.  ``forward`` and ``ddim_sample`` do not check (the checksum reads all
+        400 MB of parameters at width 1024), so call this after editing ``.data`` by hand; ``save_diffusion_samples``
+        calls it itself."""
+        if next(self.parameters()).device.type == "cuda":
+            self._checksum = params_checksum(self)
+        return self
 
     def _release(self):
         if self._handle is not None:
@@ -93,7 +103,8 @@ class DiffusionPriorFiLM(nn.Module):
         if dev.type != "cuda":
             raise RuntimeError("toycrystals_b200 runs on a CUDA (B200, sm_100a) device only; move the model with "
                                ".to('cuda') — there is no CPU fallback (use the reference package for --device cpu)")
-        key = (dev, self.precision, self.use_graph, self._sched_key, tuple((p.data_ptr(), p._version) for p in ps))
+        key = (dev, self.precision, self.use_graph, self._sched_key, tuple((p.data_ptr(), p._version) for p in ps),
+               self._checksum)
         if self._handle is not None and key == self._handle_key:
             return self._handle
         self._release()
@@ -232,7 +243,7 @@ def save_diffusion_samples(vae, prior: DiffusionPriorFiLM, sched: DiffusionSched
                            ddim_steps: int = 50) -> None:
     """Make a 6x6 grid, cycling lattice types, sweeping theta in [0, pi/3] (reference signature and conditions)."""
     vae.eval()
-    prior.eval()
+    prior.eval().refresh()   # the training loop may have updated the weights through .data
     device = torch.device(device)
     y_cat = torch.tensor([i % vae.n_types for i in range(n)], device=device, dtype=torch.int64)
     thetas = torch.linspace(0.0, theta_max, steps=n, device=device)

@@ -160,13 +160,10 @@ class CondUNetTiny(nn.Module):
                 self._fuse_gn)
 
     def weights_checksum(self) -> Tuple[int, float]:
-        """Device-side checksum of all parameters (bit pattern sum + sum of squares): catches in-place updates made through
-        ``.data`` (the training loop's EMA update, scripts/train_sde_score_model.py:239-240), which do not bump
-        ``_version``.  One small reduction and a host read."""
-        flat = torch.cat([p.detach().reshape(-1) for p in self.parameters()])
-        a = flat.view(torch.int32).sum(dtype=torch.int64)
-        b = (flat.double() ** 2).sum()
-        return int(a.item()), float(b.item())
+        """Device-side checksum of all parameters: catches in-place updates made through ``.data`` (the training loop's
+        EMA update, scripts/train_sde_score_model.py:239-240), which do not bump ``_version``.  One small reduction and a
+        host read."""
+        return params_checksum(self)
 
     def refresh(self) -> "CondUNetTiny":
         """Re-read the parameters on the next call if they changed behind autograd's back (``p.data.mul_(...)``).
@@ -237,6 +234,14 @@ class CondUNetTiny(nn.Module):
     # -- reference surface --------------------------------------------------------------------------
     def forward(self, x_t: torch.Tensor, t: torch.Tensor, y_cat: torch.Tensor, y_cont: torch.Tensor) -> torch.Tensor:
         return _score(self, x_t, t, y_cat, y_cont, 0.0)
+
+
+def params_checksum(module: nn.Module) -> Tuple[int, float]:
+    """Bit pattern sum + sum of squares of all of a module's (fp32) parameters, computed on their device."""
+    flat = torch.cat([p.detach().reshape(-1) for p in module.parameters()])
+    a = flat.view(torch.int32).sum(dtype=torch.int64)
+    b = (flat.double() ** 2).sum()
+    return int(a.item()), float(b.item())
 
 
 _adopted: "Dict[int, Tuple[object, CondUNetTiny]]" = {}
