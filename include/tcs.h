@@ -13,7 +13,7 @@
  *        <- CondUNetTiny.forward  (:243-266)  and  predict_eps_cfg (:402-423)
  *   tcs_sample
  *        <- sample_probability_flow_ode (:452-504), sample_reverse_sde_euler_maruyama (:507-569),
- *           VPSDE (:273-298); also DPM-Solver++(2M), which the reference does not have
+ *           VPSDE (:273-298); also DPM-Solver++(2M) and SDE-DPM-Solver++(2M), which the reference does not have
  *   tcs_condition_grid
  *        <- save_sde_samples condition synthesis (:317-321)
  *
@@ -48,8 +48,11 @@ enum tcs_precision { TCS_FP32 = 0, TCS_BF16 = 1 };
 enum tcs_engine { TCS_ENGINE_AUTO = 0, TCS_ENGINE_SIMT = 1, TCS_ENGINE_TCGEN05 = 2 };
 /* ODE: probability-flow ODE, Heun, quadratic time grid.  SDE: reverse VP-SDE, Euler-Maruyama.
  * DPMPP_2M: DPM-Solver++(2M) (Lu et al. 2022, Algorithm 2) on the probability-flow ODE, times uniform in
- *           log-SNR, one evaluation per step, deterministic (noise must be NULL).  Not in the reference. */
-enum tcs_sampler { TCS_SAMPLER_ODE = 0, TCS_SAMPLER_SDE = 1, TCS_SAMPLER_DPMPP_2M = 2 };
+ *           log-SNR, one evaluation per step, deterministic (noise must be NULL).  Not in the reference.
+ * DPMPP_2M_SDE: SDE-DPM-Solver++(2M) (Lu et al. 2022, the SDE variant of Algorithm 2, eta = 1) on the reverse VP-SDE: the
+ *           same grid and (c0, c1) as DPMPP_2M, one evaluation per step, stochastic: z per step from `noise` or from
+ *           Philox keyed (seed, global sample index, 1 + step), as for SDE.  Not in the reference. */
+enum tcs_sampler { TCS_SAMPLER_ODE = 0, TCS_SAMPLER_SDE = 1, TCS_SAMPLER_DPMPP_2M = 2, TCS_SAMPLER_DPMPP_2M_SDE = 3 };
 
 typedef struct tcs_config {
   int32_t n_types;     /* CondUNetTiny(n_types, ...)                                  */
@@ -100,7 +103,7 @@ typedef struct tcs_sample_args {
   const int64_t* y_cat;         /* [n] */
   const float* y_cont;          /* [n,y_cont_dim] */
   const float* x_init;          /* [n,1,64,64] or NULL -> Philox N(0,1) */
-  const float* noise;           /* [steps,n,1,64,64] or NULL -> Philox N(0,1) (SDE only; NULL for DPMPP_2M) */
+  const float* noise;           /* [steps,n,1,64,64] or NULL -> Philox N(0,1) (SDE, DPMPP_2M_SDE; NULL for DPMPP_2M) */
   uint64_t seed;                /* Philox key */
   uint64_t global_index_offset; /* index of sample 0 of this call in the whole job (sharding) */
   float* x_out;                 /* [n,1,64,64] images in [0,1] */
@@ -113,7 +116,7 @@ typedef struct tcs_sample_args {
 
 int tcs_sample(tcs_handle* h, const tcs_sample_args* args, void* stream);
 
-/* Number of network evaluations tcs_sample performs: ode (Heun) 2*steps+1, sde and dpm++2m steps+1. */
+/* Number of network evaluations tcs_sample performs: ode (Heun) 2*steps+1, sde, dpm++2m and dpm++2m-sde steps+1. */
 int32_t tcs_nfe(int32_t sampler, int32_t steps);
 
 /* y_cat[i] = (offset+i) % n_types ; y_cont[i] = [0, theta_max*(offset+i)/(n_total-1), 0, ...]. */
@@ -139,6 +142,13 @@ int tcs_ode_update(tcs_handle* h, int32_t mode, float* x, float* x_pred, float* 
 int tcs_dpm_update(tcs_handle* h, float* x, float* x0_prev, const float* eps, int32_t n, float alpha, float sigma, float a,
                    float m, float c0, float c1, void* stream);
 
+/* The SDE-DPM-Solver++(2M) update kernel on its own (bit-exactness tests), in fp32 and in this order:
+ *   x0 = (x - sigma*eps)/alpha;  D = c1 == 0 ? x0 : c0*x0 + c1*x0_prev;  x <- (a*x + m*D) + g*z;  x0_prev <- x0
+ * z from `noise` [n,1,64,64] (this step only), or NULL -> Philox keyed (seed, global_index_offset + i, 1 + step). */
+int tcs_dpm_sde_update(tcs_handle* h, float* x, float* x0_prev, const float* eps, const float* noise, int32_t n,
+                       float alpha, float sigma, float a, float m, float c0, float c1, float g, uint64_t seed,
+                       uint64_t global_index_offset, int32_t step, void* stream);
+
 /* Host-side schedule, exactly as the kernels use it (for tests): ts has steps+1 entries. */
 int tcs_time_grid_host(int32_t steps, double t_end, float* ts_host);
 int tcs_schedule_host(double beta_min, double beta_max, float t, float* beta, float* alpha, float* sigma);
@@ -149,6 +159,11 @@ int tcs_schedule_host(double beta_min, double beta_max, float t, float* beta, fl
  *   (c0, c1) = (1, 0) on step 0 and, when steps < 15, on the last step; else r = h_{i-1}/h_i, (1 + 1/(2r), -1/(2r)). */
 int tcs_dpm_schedule_host(int32_t steps, double t_end, double beta_min, double beta_max, float* ts_host,
                           float* coef_host);
+/* The SDE-DPM-Solver++(2M) schedule: the same ts_host and (c0, c1) as tcs_dpm_schedule_host; coef_host [steps][5] =
+ * (a, m, c0, c1, g), in double from the fp32 times and rounded once:
+ *   a = sigma(t_{i+1})/sigma(t_i) * exp(-h), m = alpha(t_{i+1})*(-expm1(-2h)), g = sigma(t_{i+1})*sqrt(-expm1(-2h)). */
+int tcs_dpm_sde_schedule_host(int32_t steps, double t_end, double beta_min, double beta_max, float* ts_host,
+                              float* coef_host);
 
 /* Waits for the handle's enqueued work and returns its sticky status bits (then clears them):
  *   bit 0: a fused GroupNorm layer saw a pre-norm activation that may exceed the fp16 staging range; the eps / images of

@@ -1,8 +1,8 @@
 #!/usr/bin/env python3
-"""Samples/s of the DPM-Solver++(2M) sampler at 10, 20 and 50 steps against the reverse-SDE sampler at 300 steps, at the
-bench configuration (n = 1024 per job, CFG 1.5, t_end 0.005, the bench's EMA weights: default init under seed 1, bf16 on
-the tcgen05 engine).  The four jobs alternate in one process: one warm-up round, then --reps timed rounds; each job is
-timed with CUDA events and ends in a device synchronise.  The card's name, power limit and SM clock (sampled during the
+"""Samples/s of the DPM-Solver++(2M) sampler at 10, 20 and 50 steps and of its SDE form (dpm++2m-sde) at 20, 50 and 80
+steps against the reverse-SDE sampler at 300 steps, at the bench configuration (n = 1024 per job, CFG 1.5, t_end 0.005,
+the bench's EMA weights: default init under seed 1, bf16 on the tcgen05 engine).  The seven jobs alternate in one process:
+one warm-up round, then --reps timed rounds; each job is timed with CUDA events and ends in a device synchronise.  The card's name, power limit and SM clock (sampled during the
 timed rounds) are recorded in the same run.
 
 Also reported, for information only (no gate): the pre-clamp x0_hat rel-L2 between dpm++2m at 50 steps and the Heun ODE
@@ -30,9 +30,10 @@ from toycrystals_b200.models import sde_score_model as shim  # noqa: E402
 from bench import ClockSampler  # noqa: E402
 
 N, CFG, T_END, SEED = 1024, 1.5, 0.005, 1234
-JOBS = [("dpm++2m", 10), ("dpm++2m", 20), ("dpm++2m", 50), ("sde", 300)]
-FNS = {"dpm++2m": shim.sample_dpmpp_2m, "sde": shim.sample_reverse_sde_euler_maruyama}
-SAMPLER_IDS = {"dpm++2m": _cabi.SAMPLER_DPMPP_2M, "ode": _cabi.SAMPLER_ODE}
+JOBS = [("dpm++2m", 10), ("dpm++2m", 20), ("dpm++2m", 50), ("dpm++2m-sde", 20), ("dpm++2m-sde", 50),
+        ("dpm++2m-sde", 80), ("sde", 300)]
+SAMPLER_IDS = {"dpm++2m": _cabi.SAMPLER_DPMPP_2M, "dpm++2m-sde": _cabi.SAMPLER_DPMPP_2M_SDE, "ode": _cabi.SAMPLER_ODE,
+               "sde": _cabi.SAMPLER_SDE}
 
 
 def gpu_info():
@@ -77,8 +78,8 @@ def main():
     yc, yk = shim.condition_grid(model, N, math.pi / 3.0, dev)
 
     def job(sampler, steps):
-        return FNS[sampler](model, sde, yc, yk, (N, 1, 64, 64), n_steps=steps, guidance_scale=CFG, t_end=T_END,
-                            seed=SEED)
+        return shim._SAMPLERS[sampler](model, sde, yc, yk, (N, 1, 64, 64), n_steps=steps, guidance_scale=CFG,
+                                       t_end=T_END, seed=SEED)
 
     def timed(sampler, steps):
         torch.cuda.synchronize()
@@ -101,10 +102,9 @@ def main():
     for sampler, steps in JOBS:
         key = f"{sampler}@{steps}"
         med = statistics.median(ms[key])
-        jobs[key] = {"sampler": sampler, "steps": steps, "nfe": int(_cabi.lib().tcs_nfe(
-            _cabi.SAMPLER_DPMPP_2M if sampler == "dpm++2m" else _cabi.SAMPLER_SDE, steps)),
+        jobs[key] = {"sampler": sampler, "steps": steps, "nfe": int(_cabi.lib().tcs_nfe(SAMPLER_IDS[sampler], steps)),
             "ms_per_job": ms[key], "ms_median": med, "samples_per_sec": N / (med / 1e3),
-            "ms_per_evaluation": med / (steps + 1)}
+            "ms_per_evaluation": med / (steps + 1)}   # every job here makes steps + 1 evaluations
     base = jobs["sde@300"]["samples_per_sec"]
     for v in jobs.values():
         v["speedup_vs_sde300"] = v["samples_per_sec"] / base
@@ -123,8 +123,8 @@ def main():
     with open(args.out, "w") as f:
         json.dump(res, f, indent=1)
     for k, v in jobs.items():
-        print(f"{k:>12}: {v['samples_per_sec']:8.1f} samples/s  ({v['ms_median']:.1f} ms/job, {v['nfe']} evaluations, "
-              f"x{v['speedup_vs_sde300']:.2f} vs sde@300)")
+        print(f"{k:>16}: {v['samples_per_sec']:8.1f} samples/s  ({v['ms_median']:.1f} ms/job, {v['nfe']} evaluations, "
+              f"{v['ms_per_evaluation']:.2f} ms/evaluation, x{v['speedup_vs_sde300']:.2f} vs sde@300)")
     print(f"x0_hat rel-L2 dpm++2m@50 vs ode@300: {rel:.3e}")
     print(json.dumps({"device": res["device"], "nvidia_smi": info, "clocks": res["clocks_during_timing"]}))
 

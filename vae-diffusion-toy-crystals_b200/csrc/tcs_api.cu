@@ -1,5 +1,5 @@
 // tcs_api.cu — the C ABI (include/tcs.h): handle, weights, workspace, the score network pass,
-// the three samplers (Heun ODE, Euler-Maruyama SDE, DPM-Solver++(2M)) and their CUDA-graph replay.  No PyTorch types, no CPU fallback.
+// the four samplers (Heun ODE, Euler-Maruyama SDE, DPM-Solver++(2M) and its SDE form) and their CUDA-graph replay.  No PyTorch types, no CPU fallback.
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -55,8 +55,9 @@ struct Sched {
 
 // DPM-Solver++(2M) schedule: times uniform in log-SNR lambda = log alpha - log sigma from t = 1 to t_end (endpoints pinned),
 // stored as fp32 like time_grid_host; the coefficients of step i are computed in double from those fp32 times and rounded
-// to fp32 once.  Step 0 is first order, and so is the last step when steps < 15 (the "lower order final" rule).
-static void dpm_schedule_host(int steps, double t_end, double bmin, double bmax, float* ts, DpmCoef* k) {
+// to fp32 once.  Step 0 is first order, and so is the last step when steps < 15 (the "lower order final" rule).  The ODE
+// form (sde = false) and the SDE form (eta = 1) share the grid and (c0, c1); a, m and g are given in kernels.cuh (DpmCoef).
+static void dpm_schedule_host(int steps, double t_end, double bmin, double bmax, bool sde, float* ts, DpmCoef* k) {
   const double d = bmax - bmin;
   auto alpha = [&](double t) { return exp(-0.5 * (bmin * t + 0.5 * d * (t * t))); };
   auto sigma = [&](double t) { const double a = alpha(t); return sqrt(fmax(1.0 - a * a, 1e-8)); };
@@ -74,8 +75,16 @@ static void dpm_schedule_host(int steps, double t_end, double bmin, double bmax,
     const double t0 = ts[i], t1 = ts[i + 1];
     const double h = lambda(t1) - lambda(t0);
     DpmCoef c;
-    c.a = static_cast<float>(sigma(t1) / sigma(t0));
-    c.m = static_cast<float>(alpha(t1) * -expm1(-h));
+    if (sde) {
+      const double e2 = -expm1(-2.0 * h);   // 1 - exp(-2h)
+      c.a = static_cast<float>(sigma(t1) / sigma(t0) * exp(-h));
+      c.m = static_cast<float>(alpha(t1) * e2);
+      c.g = static_cast<float>(sigma(t1) * sqrt(e2));
+    } else {
+      c.a = static_cast<float>(sigma(t1) / sigma(t0));
+      c.m = static_cast<float>(alpha(t1) * -expm1(-h));
+      c.g = 0.0f;
+    }
     if (i == 0 || (i == steps - 1 && steps < 15)) {
       c.c0 = 1.0f; c.c1 = 0.0f;
     } else {
@@ -878,14 +887,24 @@ int tcs_schedule_host(double bmin, double bmax, float t, float* beta, float* alp
   if (sigma) *sigma = s.sigma(t);
   return TCS_OK;
 }
-int tcs_dpm_schedule_host(int32_t steps, double t_end, double bmin, double bmax, float* ts, float* coef) {
-  if (steps < 1 || !ts || !coef) return fail(TCS_ERR_BAD_ARGUMENT, "tcs_dpm_schedule_host: steps >= 1, ts and coef required");
-  if (!(t_end > 0.0 && t_end < 1.0)) return fail(TCS_ERR_BAD_ARGUMENT, "tcs_dpm_schedule_host: t_end must be in (0,1)");
-  if (!(bmin > 0.0 && bmax >= bmin)) return fail(TCS_ERR_BAD_ARGUMENT, "tcs_dpm_schedule_host: need 0 < beta_min <= beta_max");
+// Both host schedules: rows of `width` floats, (a, m, c0, c1) for the ODE form and (a, m, c0, c1, g) for the SDE form.
+static int dpm_schedule_rows(const char* fn, bool sde, int32_t steps, double t_end, double bmin, double bmax, float* ts,
+                             float* coef) {
+  const std::string name(fn);
+  if (steps < 1 || !ts || !coef) return fail(TCS_ERR_BAD_ARGUMENT, name + ": steps >= 1, ts and coef required");
+  if (!(t_end > 0.0 && t_end < 1.0)) return fail(TCS_ERR_BAD_ARGUMENT, name + ": t_end must be in (0,1)");
+  if (!(bmin > 0.0 && bmax >= bmin)) return fail(TCS_ERR_BAD_ARGUMENT, name + ": need 0 < beta_min <= beta_max");
   std::vector<DpmCoef> k(steps);
-  dpm_schedule_host(steps, t_end, bmin, bmax, ts, k.data());
-  memcpy(coef, k.data(), sizeof(DpmCoef) * steps);
+  dpm_schedule_host(steps, t_end, bmin, bmax, sde, ts, k.data());
+  const int width = sde ? 5 : 4;
+  for (int i = 0; i < steps; ++i) memcpy(coef + static_cast<size_t>(i) * width, &k[i], sizeof(float) * width);
   return TCS_OK;
+}
+int tcs_dpm_schedule_host(int32_t steps, double t_end, double bmin, double bmax, float* ts, float* coef) {
+  return dpm_schedule_rows("tcs_dpm_schedule_host", false, steps, t_end, bmin, bmax, ts, coef);
+}
+int tcs_dpm_sde_schedule_host(int32_t steps, double t_end, double bmin, double bmax, float* ts, float* coef) {
+  return dpm_schedule_rows("tcs_dpm_sde_schedule_host", true, steps, t_end, bmin, bmax, ts, coef);
 }
 
 int tcs_create(tcs_handle** out, const tcs_config* cfg) {
@@ -1226,9 +1245,11 @@ int tcs_ode_update(tcs_handle* h, int32_t mode, float* x, float* x_pred, float* 
   return leave(h, user);
 }
 
-int tcs_dpm_update(tcs_handle* h, float* x, float* x0_prev, const float* eps, int32_t n, float alpha, float sigma, float a,
-                   float m, float c0, float c1, void* stream) {
-  if (!h || !x || !x0_prev || !eps || n < 0) return fail(TCS_ERR_BAD_ARGUMENT, "tcs_dpm_update: bad argument");
+// One DPM-Solver++(2M) update, either form, from caller-given coefficients (the two test hooks below).
+static int dpm_update(tcs_handle* h, const char* fn, int mode, float* x, float* x0_prev, const float* eps,
+                      const float* noise, int32_t n, float alpha, float sigma, const DpmCoef& coef, uint64_t seed,
+                      uint64_t gidx0, int32_t step, void* stream) {
+  if (!h || !x || !x0_prev || !eps || n < 0 || step < 0) return fail(TCS_ERR_BAD_ARGUMENT, std::string(fn) + ": bad argument");
   if (n == 0) return TCS_OK;
   TCS_CUDA(cudaSetDevice(h->cfg.device));
   cudaStream_t user = static_cast<cudaStream_t>(stream);
@@ -1240,17 +1261,36 @@ int tcs_dpm_update(tcs_handle* h, float* x, float* x0_prev, const float* eps, in
   memset(c, 0, sizeof(StepCoef));
   c->alpha = alpha; c->sigma = sigma;
   DpmCoef* k = reinterpret_cast<DpmCoef*>(c + 1);
-  *k = DpmCoef{a, m, c0, c1};
+  *k = coef;
+  int* hs = reinterpret_cast<int*>(c + 2);
+  *hs = step;
   TCS_CUDA(cudaMemcpyAsync(h->coef.p, c, sizeof(StepCoef), cudaMemcpyHostToDevice, h->stream));
   TCS_CUDA(cudaMemcpyAsync(h->dpm_coef.p, k, sizeof(DpmCoef), cudaMemcpyHostToDevice, h->stream));
+  TCS_CUDA(cudaMemcpyAsync(h->step_ctr.p, hs, 4, cudaMemcpyHostToDevice, h->stream));
   TCS_CUDA(cudaEventRecord(h->ev_pinned, h->stream));
   StepArgs s{};
   s.coef = h->coef.as<StepCoef>(); s.dpm = h->dpm_coef.as<DpmCoef>();
-  s.step_ptr = nullptr; s.row_off = 0;
-  s.mode = STEP_DPM2M; s.x = x; s.d0 = x0_prev; s.eps = eps; s.n = n;
+  s.step_ptr = h->step_ctr.as<int>();
+  s.row_off = -step;   // row 0 regardless of the step word used for the Philox stream
+  s.mode = mode; s.x = x; s.d0 = x0_prev; s.eps = eps; s.n = n;
+  s.noise = noise; s.noise_step_stride = 0;   // injected noise is for this step only (stride 0)
+  s.seed = seed; s.gidx0 = gidx0;
   ++h->launches;
   TCS_CHECK(launch_step(s, h->stream));
   return leave(h, user);
+}
+
+int tcs_dpm_update(tcs_handle* h, float* x, float* x0_prev, const float* eps, int32_t n, float alpha, float sigma, float a,
+                   float m, float c0, float c1, void* stream) {
+  return dpm_update(h, "tcs_dpm_update", STEP_DPM2M, x, x0_prev, eps, nullptr, n, alpha, sigma, DpmCoef{a, m, c0, c1, 0.f},
+                    0, 0, 0, stream);
+}
+
+int tcs_dpm_sde_update(tcs_handle* h, float* x, float* x0_prev, const float* eps, const float* noise, int32_t n,
+                       float alpha, float sigma, float a, float m, float c0, float c1, float g, uint64_t seed,
+                       uint64_t gidx0, int32_t step, void* stream) {
+  return dpm_update(h, "tcs_dpm_sde_update", STEP_DPM2M_SDE, x, x0_prev, eps, noise, n, alpha, sigma,
+                    DpmCoef{a, m, c0, c1, g}, seed, gidx0, step, stream);
 }
 
 int tcs_sample(tcs_handle* h, const tcs_sample_args* args, void* stream) {
@@ -1259,8 +1299,9 @@ int tcs_sample(tcs_handle* h, const tcs_sample_args* args, void* stream) {
   const tcs_sample_args& A = *args;
   if (!(A.t_end > 0.0 && A.t_end < 1.0))
     return fail(TCS_ERR_BAD_ARGUMENT, "t_end must be in (0,1), got " + std::to_string(A.t_end));
-  if (A.sampler != TCS_SAMPLER_ODE && A.sampler != TCS_SAMPLER_SDE && A.sampler != TCS_SAMPLER_DPMPP_2M)
-    return fail(TCS_ERR_BAD_ARGUMENT, "Unknown sampler. Use 'ode', 'sde' or 'dpm++2m'.");
+  if (A.sampler != TCS_SAMPLER_ODE && A.sampler != TCS_SAMPLER_SDE && A.sampler != TCS_SAMPLER_DPMPP_2M &&
+      A.sampler != TCS_SAMPLER_DPMPP_2M_SDE)
+    return fail(TCS_ERR_BAD_ARGUMENT, "Unknown sampler. Use 'ode', 'sde', 'dpm++2m' or 'dpm++2m-sde'.");
   if (A.sampler == TCS_SAMPLER_DPMPP_2M && A.noise)
     return fail(TCS_ERR_BAD_ARGUMENT, "tcs_sample: the dpm++2m sampler is deterministic; noise must be NULL");
   if (A.n < 0 || A.steps < 0) return fail(TCS_ERR_BAD_ARGUMENT, "tcs_sample: n and steps must be >= 0");
@@ -1269,10 +1310,12 @@ int tcs_sample(tcs_handle* h, const tcs_sample_args* args, void* stream) {
   const int n = A.n, steps = A.steps;
   const int dup = A.guidance > 0.f ? 2 : 1;
   const bool ode = A.sampler == TCS_SAMPLER_ODE;
-  const bool dpm = A.sampler == TCS_SAMPLER_DPMPP_2M;
+  const bool dpm_sde = A.sampler == TCS_SAMPLER_DPMPP_2M_SDE;
+  const bool dpm = A.sampler == TCS_SAMPLER_DPMPP_2M || dpm_sde;
   const Sched sc = A.beta_max > 0.0 ? Sched{A.beta_min, A.beta_max} : Sched{h->cfg.beta_min, h->cfg.beta_max};
   if (dpm && !(sc.bmin > 0.0 && sc.bmax >= sc.bmin))
-    return fail(TCS_ERR_BAD_ARGUMENT, "tcs_sample: the dpm++2m sampler needs 0 < beta_min <= beta_max");
+    return fail(TCS_ERR_BAD_ARGUMENT, std::string("tcs_sample: the ") + (dpm_sde ? "dpm++2m-sde" : "dpm++2m") +
+                                          " sampler needs 0 < beta_min <= beta_max");
   cudaStream_t user = static_cast<cudaStream_t>(stream);
   TCS_CHECK(enter(h, user));
   cudaStream_t st = h->stream;
@@ -1292,7 +1335,7 @@ int tcs_sample(tcs_handle* h, const tcs_sample_args* args, void* stream) {
   DpmCoef* hk = reinterpret_cast<DpmCoef*>(hc + steps + 2);
   float* hts = dpm ? reinterpret_cast<float*>(hk + steps + 1) : reinterpret_cast<float*>(hc + steps + 2);
   if (dpm) {
-    if (steps >= 1) dpm_schedule_host(steps, A.t_end, sc.bmin, sc.bmax, hts, hk);
+    if (steps >= 1) dpm_schedule_host(steps, A.t_end, sc.bmin, sc.bmax, dpm_sde, hts, hk);
     else hts[0] = 1.0f;   // no step: the projection of x_T at t = 1, as for the other samplers
   } else if (steps >= 1) {
     time_grid_host(steps, A.t_end, hts);
@@ -1335,12 +1378,12 @@ int tcs_sample(tcs_handle* h, const tcs_sample_args* args, void* stream) {
     return a;
   };
   auto enqueue_step = [&]() -> int {
-    if (!ode) {   // SDE and DPM-Solver++(2M): one evaluation per step
+    if (!ode) {   // SDE and both DPM-Solver++(2M) forms: one evaluation per step
       TCS_CHECK(trace_copy(h, A.trace_x, x, sp, 1, 0, n, st));
       TCS_CHECK(forward_all(h, x, cvec, tvec, 0, sp, 0, n, dup, A.guidance, eps, st));
       TCS_CHECK(trace_copy(h, A.trace_eps, eps, sp, 1, 0, n, st));
       ++h->launches;
-      TCS_CHECK(launch_step(step_args(dpm ? STEP_DPM2M : STEP_SDE, 0), st));
+      TCS_CHECK(launch_step(step_args(dpm_sde ? STEP_DPM2M_SDE : dpm ? STEP_DPM2M : STEP_SDE, 0), st));
     } else {
       TCS_CHECK(trace_copy(h, A.trace_x, x, sp, 2, 0, n, st));
       TCS_CHECK(forward_all(h, x, cvec, tvec, 0, sp, 0, n, dup, A.guidance, eps, st));

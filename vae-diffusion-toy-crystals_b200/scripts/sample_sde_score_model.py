@@ -1,8 +1,9 @@
 #!/usr/bin/env python3
 """Same command line as the reference's scripts/sample_sde_score_model.py (:30-131): same flags,
 defaults, checkpoint layout ({"config","model",["ema"]}), default output name and final print.
-Additions: --precision {bf16,fp32}, --out-tensor (dump all n samples as a .pt tensor) and --sampler dpm++2m
-(DPM-Solver++(2M): one network evaluation per step; 20 steps is the usual choice).
+Additions: --precision {bf16,fp32}, --out-tensor (dump all n samples as a .pt tensor), --sampler dpm++2m
+(DPM-Solver++(2M): one network evaluation per step; 20 steps is the usual choice) and --sampler dpm++2m-sde
+(SDE-DPM-Solver++(2M): stochastic, second order, one evaluation per step).
 
     python scripts/sample_sde_score_model.py --out-dir runs/sde --steps 300 --cfg 1.5 \
         --t-end 0.005 --sampler sde --use-ema 1

@@ -8,6 +8,7 @@ error behaviour — with every computation done by libtcs.so (hand-written sm_10
     sample_probability_flow_ode        (:452-504)  -> tcs_sample (Heun)
     sample_reverse_sde_euler_maruyama  (:507-569)  -> tcs_sample (Euler-Maruyama)
     sample_dpmpp_2m                    (addition)  -> tcs_sample (DPM-Solver++(2M), one evaluation per step)
+    sample_dpmpp_2m_sde                (addition)  -> tcs_sample (SDE-DPM-Solver++(2M), one evaluation per step)
     save_sde_samples                   (:301-355)  condition grid + sampler + 6x6 PNG
 
 PyTorch is used for device memory, streams and the state-dict container only.  There is no CPU
@@ -380,7 +381,7 @@ def _sample(model: CondUNetTiny, sde: VPSDE, y_cat, y_cont, img_shape, n_steps, 
     # reproduces a run and a sharded job equals the unsharded one
     x_init = None if x_init is None else _as_f32(x_init, device)
     noise_t = None
-    if sampler == _cabi.SAMPLER_SDE:
+    if sampler in (_cabi.SAMPLER_SDE, _cabi.SAMPLER_DPMPP_2M_SDE):
         if isinstance(noise, str) and noise == "torch":
             # reference-identical consumption of the global generator: one randn_like per step
             noise_t = (torch.stack([torch.randn((B, 1, 64, 64), device=device) for _ in range(n_steps)])
@@ -454,7 +455,25 @@ def sample_dpmpp_2m(model: CondUNetTiny, sde: VPSDE, y_cat: torch.Tensor, y_cont
                    x_init=x_init, seed=seed, global_index_offset=global_index_offset, return_trace=return_trace)
 
 
-_SAMPLERS = {"ode": sample_probability_flow_ode, "sde": sample_reverse_sde_euler_maruyama, "dpm++2m": sample_dpmpp_2m}
+@torch.no_grad()
+def sample_dpmpp_2m_sde(model: CondUNetTiny, sde: VPSDE, y_cat: torch.Tensor, y_cont: torch.Tensor,
+                        img_shape: Tuple[int, int, int, int], n_steps: int = 80, guidance_scale: float = 0.0,
+                        t_end: float = 1e-3, *, x_init=None, noise=None, seed=None, global_index_offset: int = 0,
+                        return_trace: bool = False):
+    """Stochastic sampler: SDE-DPM-Solver++(2M) (Lu et al. 2022, the SDE variant of Algorithm 2, eta = 1) on the
+    reverse VP-SDE, on the grid and with the first-order rows of ``sample_dpmpp_2m``, one network evaluation per step,
+    final x0 projection; returns [B,1,64,64] in [0,1].  n_steps + 1 evaluations in all.  It solves the linear part and
+    the noise exactly and is second order in the data term, where Euler-Maruyama is first order.  ``noise`` as for
+    ``sample_reverse_sde_euler_maruyama`` (None = Philox keyed (seed, global sample index, 1 + step), "torch", or a
+    tensor [n_steps,B,1,64,64]); ``x_init`` / ``seed`` / ``global_index_offset`` / ``return_trace`` as for the other
+    samplers; the trace has the SDE sampler's layout."""
+    return _sample(model, sde, y_cat, y_cont, img_shape, n_steps, guidance_scale, t_end, _cabi.SAMPLER_DPMPP_2M_SDE,
+                   x_init=x_init, noise=noise, seed=seed, global_index_offset=global_index_offset,
+                   return_trace=return_trace)
+
+
+_SAMPLERS = {"ode": sample_probability_flow_ode, "sde": sample_reverse_sde_euler_maruyama, "dpm++2m": sample_dpmpp_2m,
+             "dpm++2m-sde": sample_dpmpp_2m_sde}
 
 
 def condition_grid(model: CondUNetTiny, n: int, theta_max: float, device, offset: int = 0, n_total: Optional[int] = None):
@@ -497,7 +516,7 @@ def save_sde_samples(model: CondUNetTiny, sde: VPSDE, out_path: str, device: tor
     model.eval()
     device = torch.device(device)
     if sampler not in _SAMPLERS:
-        raise ValueError(f"Unknown sampler='{sampler}'. Use 'ode', 'sde' or 'dpm++2m'.")
+        raise ValueError(f"Unknown sampler='{sampler}'. Use 'ode', 'sde', 'dpm++2m' or 'dpm++2m-sde'.")
     model = adopt(model)
     y_cat, y_cont = condition_grid(model, n, theta_max, device)
     fn = _SAMPLERS[sampler]
