@@ -85,7 +85,6 @@ def debug_conv(engine, precision, in0, in1, w, b, ksize, stride, epi):
 
 
 ATTN_DBG_FLOATS = 256 * 192 + 256 * 576 + 256 * 192 + 256 * 4
-ATTN_PROF_SLOTS = 96   # clock64 stamps (int64) of the control lane and of one worker lane follow the float dump
 
 
 def debug_attn_block(x, gn_w, gn_b, qkv_w, qkv_b, proj_w, proj_b, want_dbg=False):
@@ -94,7 +93,7 @@ def debug_attn_block(x, gn_w, gn_b, qkv_w, qkv_b, proj_w, proj_b, want_dbg=False
     L = _cabi.lib()
     B = x.shape[0]
     out = torch.full((B, 16, 16, 192), float("nan"), device="cuda")
-    dbg = torch.zeros((ATTN_DBG_FLOATS + 2 * 2 * ATTN_PROF_SLOTS,), device="cuda") if want_dbg else None
+    dbg = torch.zeros((ATTN_DBG_FLOATS,), device="cuda") if want_dbg else None
     ts = [t.contiguous().float().cuda() for t in (x, gn_w, gn_b, qkv_w.reshape(576, 192), qkv_b, proj_w.reshape(192, 192), proj_b)]
     torch.cuda.synchronize()
     _cabi.check(L.tcs_debug_attn_block(B, *[t.data_ptr() for t in ts], out.data_ptr(),
@@ -104,8 +103,7 @@ def debug_attn_block(x, gn_w, gn_b, qkv_w, qkv_b, proj_w, proj_b, want_dbg=False
     if dbg is not None:
         o = [0, 256 * 192, 256 * 192 + 256 * 576, 256 * 192 + 256 * 576 + 256 * 192]
         d = {"xn": dbg[o[0]:o[1]].reshape(256, 192), "qkv": dbg[o[1]:o[2]].reshape(256, 576),
-             "y": dbg[o[2]:o[3]].reshape(256, 192), "l": dbg[o[3]:ATTN_DBG_FLOATS].reshape(256, 4),
-             "prof": dbg[ATTN_DBG_FLOATS:].view(torch.int64).reshape(2, ATTN_PROF_SLOTS).cpu()}
+             "y": dbg[o[2]:o[3]].reshape(256, 192), "l": dbg[o[3]:ATTN_DBG_FLOATS].reshape(256, 4)}
     return out, d
 
 

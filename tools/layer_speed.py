@@ -1,5 +1,5 @@
 #!/usr/bin/env python3
-"""Per-conv-layer TFLOP/s of one network pass (tcs_score_profiled), for timing experiments."""
+"""Per-conv-layer TFLOP/s of one network pass (tcs_score_profiled)."""
 import json
 import os
 import sys
@@ -16,5 +16,5 @@ torch.manual_seed(1)
 m = shim.CondUNetTiny(4, 4, 96, 128, 8, 8, precision="bf16").cuda().eval()
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 128   # samples per pass (images = 2n); bench.py uses 128
 k = bench.profile_kernels(m, shim.VPSDE(0.1, 30.0), torch.device("cuda", 0), n)
-print(os.environ.get("TCS_DEBUG", "0"), round(k["conv_tflops"], 1), round(k["conv_ms"], 3), round(k["conv_share"], 3),
+print(round(k["conv_tflops"], 1), round(k["conv_ms"], 3), round(k["conv_share"], 3),
       json.dumps(k["per_layer"]))

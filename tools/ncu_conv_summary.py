@@ -1,12 +1,10 @@
 #!/usr/bin/env python3
 """Summarise an `ncu --set full` capture of one network pass of the tcgen05 conv family into profiles/*.json.
 
-  ncu --set full --clock-control none --import-source on -k regex:conv_tc_kernel -s 16 -c 16 \
-      -o gpurun_out/prof_conv python tools/ncu_target.py 128 1
-  python tools/ncu_conv_summary.py gpurun_out/prof_conv.ncu-rep profiles/r1_conv_ncu_full.json
+  python tools/ncu_conv_summary.py <capture>.ncu-rep profiles/r1_conv_ncu_full.json
 
-`tools/ncu_target.py 128 1` runs 4 network passes of 256 images (CFG-doubled n = 128) with 16 conv_tc launches each
-(15 layers + the output conv), so `-s 16 -c 16` is exactly the second pass.  bench.py reads `traffic_bytes_per_pass`.
+The committed captures ran 4 network passes of 256 images (CFG-doubled n = 128) with 16 conv_tc launches each
+(15 layers + the output conv) and kept `-s 16 -c 16`, exactly the second pass.  bench.py reads `traffic_bytes_per_pass`.
 """
 import csv
 import io

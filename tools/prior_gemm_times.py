@@ -1,5 +1,5 @@
 #!/usr/bin/env python3
-"""fc1 / fc2 / LN+FiLM / tail kernel times of the latent prior (tcs_prior_profile), n rows.  Env switches of linear_tc apply."""
+"""fc1 / fc2 / LN+FiLM / tail kernel times of the latent prior (tcs_prior_profile), n rows."""
 import ctypes as C
 import os
 import sys
@@ -17,15 +17,10 @@ prior = pshim.DiffusionPriorFiLM(32, 4, 4, 64, 1024, 8, 64, precision="bf16").cu
 sched = pshim.DiffusionSchedule.linear(1000, 1e-4, 0.05, torch.device("cuda"))
 y_cat = (torch.arange(n, device="cuda") % 4).to(torch.int64)
 y_cont = torch.zeros((n, 4), device="cuda")
-if not (int(os.environ.get("TCS_LT_DEBUG", "0")) & 2):
-    sched.ddim_sample(prior, y_cat, y_cont, n_steps=3, seed=1)
-else:
-    os.environ["TCS_LT_DEBUG_SAVE"] = os.environ.pop("TCS_LT_DEBUG")
-    sched.ddim_sample(prior, y_cat, y_cont, n_steps=3, seed=1)
-    os.environ["TCS_LT_DEBUG"] = os.environ["TCS_LT_DEBUG_SAVE"]
+sched.ddim_sample(prior, y_cat, y_cont, n_steps=3, seed=1)
 torch.cuda.synchronize()
 ms = (C.c_float * 4)()
 _cabi.check(_cabi.lib().tcs_prior_profile(prior.engine_handle(sched), n, 50, ms))
 fl = 2.0 * n * 1024 * 4096
-print(f"n={n} env={ {k: v for k, v in os.environ.items() if k.startswith('TCS_')} } fc1 {ms[0]*1e3:.1f} us ({fl/ms[0]/1e9:.0f} TF)  "
+print(f"n={n} fc1 {ms[0]*1e3:.1f} us ({fl/ms[0]/1e9:.0f} TF)  "
       f"fc2 {ms[1]*1e3:.1f} us ({fl/ms[1]/1e9:.0f} TF)  lnf {ms[2]*1e3:.1f} us  tail {ms[3]*1e3:.1f} us")

@@ -22,7 +22,6 @@ SOURCES = ["tcs_api.cu", "conv_tc.cu", "kernels_simt.cu", "kernels_split.cu", "k
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
          "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr", "-Xptxas", "-v"]
-FLAGS += os.environ.get("TCS_NVCC_EXTRA", "").split()   # experiments only, e.g. -DTCS_KERNEL_PROFILE=1 (build with --force)
 
 
 def source_hash() -> str:

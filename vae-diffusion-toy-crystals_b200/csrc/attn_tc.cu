@@ -172,10 +172,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(AT_THREADS, 1) attn_
   cluster.sync();   // the peer is running and its barriers are initialised: its shared memory may be written from here on
 
   const int ncl = gridDim.x >> 1, cl = blockIdx.x >> 1;
-  if (p.stagger > 0) {   // de-synchronise the clusters: their memory phases (image boundaries) then hit L2 / HBM at different times
-    const long long t0 = clock64(), d = static_cast<long long>(cl & 15) * p.stagger;
-    while (clock64() - t0 < d) { }
-  }
   // phase parities, one set per waiting role (control lane / workers); every wait flips its own bit
   uint32_t ph_w = 0, ph_qkv = 0, ph_s = 0, ph_o = 0, ph_y = 0, ph_kl = 0, ph_vl = 0, ph_kf = 0, ph_vf = 0, ph_kfree = 0,
            ph_vfree = 0, ph_od = 0, ph_p = 0, ph_x = 0, ph_r = 0;
@@ -208,12 +204,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(AT_THREADS, 1) attn_
   if (ctrl && lane == 0 && cl < p.B) fetch_x(cl);
 
   for (int img = cl; img < p.B; img += ncl) {
-    // clock64 phase profile (tests / tuning only): control lane and the first worker lane of CTA 0, second image of its loop
-    long long* prof = (p.dbg && blockIdx.x == 0 && img == cl + ncl && (tid == 0 || tid == 32))
-                          ? reinterpret_cast<long long*>(p.dbg + ATTN_DBG_FLOATS) + (tid ? ATTN_PROF_SLOTS : 0) : nullptr;
-    int prof_i = 0;
-#define AT_PROF() { if (prof && prof_i < ATTN_PROF_SLOTS) prof[prof_i++] = clock64(); }
-    AT_PROF();
     __nv_bfloat16* ob = p.out + static_cast<size_t>(img) * AT_PIMG;
     float* dbg = (p.dbg && img == 0) ? p.dbg : nullptr;
     // ---- phase 0 (all threads): GroupNorm statistics over both CTAs' halves, Xn normalised in place -----------------
@@ -288,7 +278,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(AT_THREADS, 1) attn_
       ptx::tc_fence_before();
       ptx::bulk_wait_read<0>();   // the previous image's output rows have left the staging rows (= the K / V regions)
       __syncthreads();
-      AT_PROF();   // phase 0 done
     }
     if (ctrl) {
       // ================= control lane: every MMA, the weight loads, the K / V pushes to the peer =====================
@@ -320,7 +309,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(AT_THREADS, 1) attn_
         };
         issue_qkv();
         load_weights(1);
-        AT_PROF();   // c: qkv_0 done, W_1 requested
         for (int h = 0; h < N_HEADS; ++h) {
           // K rows (and Q' in tensor memory) of my tokens are stored: push my K rows, then S as soon as the peer's are here
           ptx::mbar_wait(b_kl, ph_kl); ph_kl ^= 1;
@@ -328,7 +316,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(AT_THREADS, 1) attn_
           bulk_push_to_peer(sb + K_OFF + rank * 16384, 16384, b_kf, peer);
           ptx::mbar_wait(b_kf, ph_kf); ph_kf ^= 1;
           ptx::mbar_expect_tx(b_kf, 16384);
-          AT_PROF();   // c: all keys here
           ptx::tc_fence_after();
           {
             const uint32_t idesc = make_idesc(128, 256);
@@ -337,14 +324,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(AT_THREADS, 1) attn_
             for (int ks = 0; ks < 3; ++ks) ptx::umma_bf16_ts(tmem + S_COL, tmem + Q_COL + 8 * ks, kd + 2 * ks, idesc, ks ? 1u : 0u);
             ptx::umma_commit(b_s);
           }
-          AT_PROF();   // c: S issued
           ptx::mbar_wait(b_vl, ph_vl); ph_vl ^= 1;
           if (h > 0) { ptx::mbar_wait(b_vfree, ph_vfree); ph_vfree ^= 1; }
           bulk_push_to_peer(sb + V_OFF + rank * 16384, 16384, b_vf, peer);
           if (h < N_HEADS - 1) issue_qkv();   // next head's projection runs under this head's softmax (qkv_h has been read)
           ptx::mbar_wait(b_s, ph_s); ph_s ^= 1;                       // S_h complete: the peer may overwrite its K rows here
           if (h < N_HEADS - 1) mbar_arrive_peer(b_kfree, peer);
-          AT_PROF();   // c: V pushed, next qkv issued
           ptx::mbar_wait(b_vf, ph_vf); ph_vf ^= 1;
           ptx::mbar_expect_tx(b_vf, 16384);
           {
@@ -363,7 +348,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(AT_THREADS, 1) attn_
             ph_p ^= 1;
             ptx::umma_commit(b_o);
           }
-          AT_PROF();   // c: PV issued
           if (h < N_HEADS - 1) load_weights(h + 2);                    // qkv_{h+1} complete -> W_{h+2} / Wproj
           ptx::mbar_wait(b_o, ph_o); ph_o ^= 1;                       // O_h complete: the S / P columns and V rows are free
           if (h < N_HEADS - 1) {
@@ -375,7 +359,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(AT_THREADS, 1) attn_
             for (int kb = 0; kb < 3; ++kb)
               ptx::tma_load_4d(sb + R_OFF + kb * KBLK, &maps.x, b_r, kb * 64, 1, 1 + 8 * static_cast<int>(rank), img);
           }
-          AT_PROF();   // c: head done
         }
         // projection
         ptx::mbar_wait(b_od, ph_od); ph_od ^= 1;
@@ -392,14 +375,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(AT_THREADS, 1) attn_
           }
           ptx::umma_commit(b_y);
         }
-        AT_PROF();   // c: projection issued
         ptx::mbar_wait(b_y, ph_y); ph_y ^= 1;
         if (img + ncl < p.B) {   // next image: raw rows into the O region (the projection has read it), first head's weights
           fetch_x(img + ncl);
           ptx::mbar_expect_tx(b_w, WH_BYTES);
           ptx::bulk_load_1d(sb + W_OFF, p.wpack, WH_BYTES, b_w);
         }
-        AT_PROF();   // c: image done
       }
       __syncwarp();
     } else {
@@ -466,11 +447,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(AT_THREADS, 1) attn_
       };
       convert_qk(0);
       convert_v(0);
-      AT_PROF();   // w: head 0 converted
       for (int h = 0; h < N_HEADS; ++h) {
         // ---- softmax over keys [128 hf, 128 hf + 128) of row `row`; P (bf16) overwrites the first half of those columns
         ptx::mbar_wait(b_s, ph_s); ph_s ^= 1;
-        AT_PROF();   // w: S ready
         ptx::tc_fence_after();
         const uint32_t sc = lane_addr + S_COL + 128 * hf;
         float m = -INFINITY;
@@ -511,13 +490,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(AT_THREADS, 1) attn_
           __syncwarp();
           if (lane == 0) ptx::mbar_arrive(b_p0 + 8 * 3);
         }
-        AT_PROF();   // w: softmax done
         // ---- next head's Q' and K rows (S_h is complete, so Q' and this CTA's K rows may be overwritten) ---------------
         if (h < N_HEADS - 1) convert_qk(h + 1);
-        AT_PROF();   // w: next q, k converted
         // ---- O_h / l -> shared memory (A operand of the projection) ----------------------------------------------------
         ptx::mbar_wait(b_o, ph_o); ph_o ^= 1;
-        AT_PROF();   // w: O ready
         ptx::tc_fence_after();
         {
           float o[24], lsum;
@@ -548,7 +524,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(AT_THREADS, 1) attn_
           __syncwarp();
           if (lane == 0) ptx::mbar_arrive(b_od);
         }
-        AT_PROF();   // w: head done
       }
       // ---- projection epilogue: y + bias + x -> bf16, in place in the staging rows (K-block layout, SWIZZLE_128B), then
       // three TMA tensor stores (+ three for the wrapped halo row); border columns are written by their own threads -------
@@ -556,7 +531,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(AT_THREADS, 1) attn_
       const long long wy = static_cast<long long>(halo_wrap16(ty)) * 18 * 192, wx = static_cast<long long>(halo_wrap16(tx)) * 192;
       __nv_bfloat16* dcol = ob + static_cast<size_t>((ty + 1) * 18 + tx + 1) * 192 + 96 * hf;
       ptx::mbar_wait(b_y, ph_y); ph_y ^= 1;
-      AT_PROF();   // w: Y ready
       ptx::tc_fence_after();
       ptx::mbar_wait(b_r, ph_r); ph_r ^= 1;
 #pragma unroll
@@ -583,7 +557,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(AT_THREADS, 1) attn_
       ptx::fence_proxy_async();
       ptx::tc_fence_before();
       worker_bar();
-      AT_PROF();   // w: output rows staged
       if (wt == 0) {
 #pragma unroll
         for (int kb = 0; kb < 3; ++kb) {
@@ -594,10 +567,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(AT_THREADS, 1) attn_
         }
         ptx::bulk_commit();
       }
-      AT_PROF();   // w: image written
     }
   }
-#undef AT_PROF
   ptx::bulk_wait_all();
   ptx::tc_fence_before();
   cluster.sync();      // no remote arrive / push may target a CTA that has exited
@@ -686,10 +657,7 @@ int launch_attn_block_tc(const AttnTcParams& p, int sm_count, cudaStream_t st) {
         mk(&maps.out_row, p.out, box1) != CUDA_SUCCESS)
       return fail(TCS_ERR_CUDA, "attn_tc: cuTensorMapEncodeTiled failed");
   }
-  AttnTcParams pp = p;
-  static const int stagger = getenv("TCS_ATTN_STAGGER") ? atoi(getenv("TCS_ATTN_STAGGER")) : 0;
-  pp.stagger = stagger;
-  attn_block_tc_kernel<<<2 * ncl, AT_THREADS, smem, st>>>(maps, pp);
+  attn_block_tc_kernel<<<2 * ncl, AT_THREADS, smem, st>>>(maps, p);
   TCS_CUDA(cudaGetLastError());
   return TCS_OK;
 }

@@ -13,16 +13,13 @@ struct AttnTcParams {
   const float* gamma;        // attn.norm.weight [192]
   const float* beta;         // attn.norm.bias [192]
   int B;
-  int stagger;               // cycles of start delay per (cluster index mod 16); 0 = none
-  float* dbg;                // tests only (or null): intermediates of image 0, see ATTN_DBG_* offsets
+  float* dbg;               // tests only (or null): intermediates of image 0, see ATTN_DBG_* offsets
 };
 
 // debug dump layout (floats): normalised input [256][192] | q,k,v + bias [256][576] | attention output y [256][192] |
 // softmax denominators [256][4]
 constexpr size_t ATTN_DBG_XN = 0, ATTN_DBG_QKV = 256 * 192, ATTN_DBG_Y = ATTN_DBG_QKV + 256 * 576,
                  ATTN_DBG_L = ATTN_DBG_Y + 256 * 192, ATTN_DBG_FLOATS = ATTN_DBG_L + 256 * 4;
-// followed by 2 x ATTN_PROF_SLOTS clock64 stamps (int64): control lane, first worker lane of CTA 0 on its second image
-constexpr int ATTN_PROF_SLOTS = 96;
 
 size_t attn_tc_wpack_bytes();
 // qkv_w [576][192], proj_w [192][192] (PyTorch [out][in] of the 1x1 convs) -> the shared-memory images the kernel

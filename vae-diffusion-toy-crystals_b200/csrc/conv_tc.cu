@@ -26,12 +26,6 @@
 #include <type_traits>
 #include <vector>
 
-// -DTCS_KERNEL_PROFILE=1 compiles the in-kernel clock64 phase profiler in (printed per layer with TCS_DEBUG=128);
-// the default build leaves it out so that it costs no registers
-#ifndef TCS_KERNEL_PROFILE
-#define TCS_KERNEL_PROFILE 0
-#endif
-
 namespace tcs {
 
 
@@ -72,7 +66,6 @@ constexpr uint32_t EPI_FUSED_BYTES = sizeof(EpiFusedSmem);
 // The G CTAs of an image wait for each other's GroupNorm partial sums (one L2 round trip when they run in lock step).
 // Co-residency of the whole grid is guaranteed by the launch (cooperative attribute, grid clamped to
 // cudaOccupancyMaxActiveClusters), so this bound only turns a protocol bug into a launch failure instead of a hang.
-// (TCS_EXCHANGE_TIMEOUT=<cycles> overrides it: instrumented ncu passes run the kernel orders of magnitude slower.)
 constexpr long long EXCHANGE_TIMEOUT_CYCLES = 1000000000LL;   // ~0.5 s
 
 __device__ __forceinline__ void st_relaxed_gpu_u64(unsigned long long* p, unsigned long long v) {
@@ -119,13 +112,9 @@ __device__ __forceinline__ void add2(float& d0, float& d1, float a0, float a1, f
       : "=f"(d0), "=f"(d1) : "f"(a0), "f"(a1), "f"(b0), "f"(b1));
 }
 __device__ __forceinline__ float tanh_fast(float x) {
-#ifdef TCS_NO_TANH
-  return x * 0.25f;   // timing experiment only: no MUFU in the fused epilogue
-#else
   float t;
   asm("tanh.approx.f32 %0, %1;" : "=f"(t) : "f"(x));
   return t;
-#endif
 }
 __device__ __forceinline__ void st_shared_u4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
   asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
@@ -148,16 +137,13 @@ template <int GEO = 0, int SB = SLAB_BUFS>
 __device__ __forceinline__ void store_padded_block(const CUtensorMap* mapO, bool use_tma, uint32_t slab, uint32_t& slab_buf,
                                                    int lane, __nv_bfloat16* obase, size_t pix, int wy, int wx, int Wp,
                                                    int ldo, int ch, int img, int y, int x, const uint32_t* pk,
-                                                   long long* tacc = nullptr, int h16 = 0,
-                                                   const CUtensorMap* mapO1 = nullptr, int geo_H = 0) {
+                                                   int h16 = 0, const CUtensorMap* mapO1 = nullptr, int geo_H = 0) {
   if (!use_tma) {
     store_with_halo(obase, pix, wy, wx, Wp, ldo, ch, pk);
     return;
   }
-  long long c0 = tacc ? clock64() : 0;
   if (lane == 0) ptx::bulk_wait_read<SB - 1>();   // the staging block about to be overwritten has been read
   __syncwarp();
-  if (tacc) { const long long c1 = clock64(); tacc[0] += c1 - c0; c0 = c1; }
   const uint32_t base = slab + (SB == 2 ? slab_buf * 2048 : 0);
   const uint32_t dst = base + lane * 64;
   const int sw = (lane >> 1) & 3;
@@ -165,7 +151,6 @@ __device__ __forceinline__ void store_padded_block(const CUtensorMap* mapO, bool
   for (int j = 0; j < 4; ++j) st_shared_u4(dst + ((j ^ sw) << 4), pk[4 * j], pk[4 * j + 1], pk[4 * j + 2], pk[4 * j + 3]);
   ptx::fence_proxy_async();
   __syncwarp();
-  if (tacc) { const long long c1 = clock64(); tacc[1] += c1 - c0; c0 = c1; }
   if (lane == 0) {   // lane 0 holds the first pixel of the block: (y, x) -> padded (y+1, x+1)
     if (GEO == 1) {
       tma_store_4d(mapO, base, ch, x + 1, y + 1, img);
@@ -183,7 +168,6 @@ __device__ __forceinline__ void store_padded_block(const CUtensorMap* mapO, bool
     ptx::bulk_commit();
   }
   __syncwarp();
-  if (tacc) { const long long c1 = clock64(); tacc[2] += c1 - c0; c0 = c1; }
   slab_buf ^= 1;
   if (wx) {   // column halo (and the corner when this pixel is also on a border row)
     uint4* d0 = reinterpret_cast<uint4*>(obase + (pix + wx) * ldo + ch);
@@ -278,8 +262,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
   const int lane = threadIdx.x & 31;
   const uint32_t smem_base = (ptx::smem_u32(smem_raw) + 1023u) & ~1023u;
   const int n_tiles = p.n_mtiles * p.n_ntiles;
-  // after the operand ring: 16 epilogue warps x 2 x 2 KB staging blocks (fp16 stash of the fused epilogue, TMA-store
-  // source of every bf16 output), then the bias
+  // after the operand ring: 16 epilogue warps x 2 x 2 KB staging blocks (TMA-store source of every bf16 output), then
+  // the bias
   const uint32_t l_ring = smem_base + (GEO == 1 ? p.a_stages * p.a_bytes : 0u);   // UPS: low-resolution windows after the window ring
   const uint32_t b_ring = l_ring + (UPS ? p.l_stages * p.l_bytes : 0u);           // geo 1: windows first, then weight stages
   const uint32_t slab_base = b_ring + p.nstage * p.stage_bytes;
@@ -316,12 +300,12 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
     if (GEO == 1) ptx::prefetch_tmap(&mapO1);
     for (int s = 0; s < p.nstage; ++s) {
       ptx::mbar_init(ptx::smem_u32(&bars.full[s]), 1);
-      ptx::mbar_init(ptx::smem_u32(&bars.empty[s]), p.issuers);     // one tcgen05.commit per issuing thread
+      ptx::mbar_init(ptx::smem_u32(&bars.empty[s]), MSUB);     // one tcgen05.commit per issuing thread
     }
     if (GEO == 1)
       for (int s = 0; s < p.a_stages; ++s) {
         ptx::mbar_init(ptx::smem_u32(&bars.fullA[s]), UPS ? 4 * CG : 1);   // UPS: one arrival per blending warp of the pair
-        ptx::mbar_init(ptx::smem_u32(&bars.emptyA[s]), p.issuers);
+        ptx::mbar_init(ptx::smem_u32(&bars.emptyA[s]), MSUB);
       }
     if (UPS)
       for (int s = 0; s < p.l_stages; ++s) {
@@ -329,7 +313,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
         ptx::mbar_init(ptx::smem_u32(&bars.emptyL[s]), 4);
       }
     for (int a = 0; a < 2; ++a) {
-      ptx::mbar_init(ptx::smem_u32(&bars.tmem_full[a]), p.issuers);
+      ptx::mbar_init(ptx::smem_u32(&bars.tmem_full[a]), MSUB);
       ptx::mbar_init(ptx::smem_u32(&bars.tmem_empty[a]), GRP_WARPS * CG);
     }
     ptx::fence_barrier_init();
@@ -384,13 +368,10 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
             if (ntile < n_tiles) issue_low(ntile, ncb);
           } else {
           ptx::mbar_wait(ptx::smem_u32(&bars.emptyA[sa]), pa ^ 1);
-          const bool stale = (p.debug & 8) && (pa || tile != static_cast<int>(blockIdx.x));   // experiment: no TMA
           if (lane == 0) {
             const uint32_t full = ptx::smem_u32(&bars.fullA[sa]);
             const uint32_t a_dst = smem_base + sa * p.a_bytes;
-            if (stale) {
-              if (CG == 1 || cta_rank == 0) ptx::mbar_arrive(full);
-            } else if (CG == 2) {
+            if (CG == 2) {
               if (cta_rank == 0) ptx::mbar_expect_tx(full, 2 * p.a_load_bytes);
               ptx::tma_load_4d_2sm(a_dst, mapA, full, cb * KB, tx * 8 * MSUB + p.base_off[src], ty * 16 + p.base_off[src], b);
             } else {
@@ -404,14 +385,11 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
           for (int kx = 0; kx < 3; ++kx, ++ks)
             for (int jb = 0; jb < b_stages_per_kx; ++jb) {
               ptx::mbar_wait(ptx::smem_u32(&bars.empty[sb]), pb ^ 1);
-              const bool stale_b = (p.debug & 8) && (pb || tile != static_cast<int>(blockIdx.x));
               if (lane == 0) {
                 const uint32_t full = ptx::smem_u32(&bars.full[sb]);
                 const uint32_t b_dst = b_ring + sb * p.stage_bytes;
                 const int row0 = ((ks * p.n_ntiles + nt) * CG + static_cast<int>(cta_rank)) * b_rows_full + jb * p.b_rows;
-                if (stale_b) {
-                  if (CG == 1 || cta_rank == 0) ptx::mbar_arrive(full);
-                } else if (CG == 2) {
+                if (CG == 2) {
                   if (cta_rank == 0) ptx::mbar_expect_tx(full, 2 * p.tb * NB * ROWB);
                   ptx::tma_load_2d_2sm(b_dst, &mapW, full, 0, row0);
                 } else {
@@ -443,12 +421,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
           for (int kyg = 0; kyg < p.KYG; ++kyg)
             for (int kx = 0; kx < p.KW; ++kx, ++ks) {
               ptx::mbar_wait(ptx::smem_u32(&bars.empty[stage]), phase ^ 1);
-              if ((p.debug & 8) && (phase || tile != static_cast<int>(blockIdx.x))) {   // experiment: stale operands, no TMA
-                if (lane == 0 && (CG == 1 || cta_rank == 0)) ptx::mbar_arrive(ptx::smem_u32(&bars.full[stage]));
-                __syncwarp();
-                if (++stage == static_cast<uint32_t>(p.nstage)) { stage = 0; phase ^= 1; }
-                continue;
-              }
               if (lane == 0) {
                 const uint32_t full = ptx::smem_u32(&bars.full[stage]);
                 const uint32_t a_dst = smem_base + stage * p.stage_bytes;
@@ -480,13 +452,13 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
             }
       }
     }
-  } else if ((warp == 1 || (warp == 2 + EPI_WARPS && p.issuers == 2)) && cta_rank == 0) {
+  } else if ((warp == 1 || (warp == 2 + EPI_WARPS && MSUB == 2)) && cta_rank == 0) {
     // ============================== MMA issuer (leader CTA only when CG == 2) ====
     // The issue loop is the critical resource of this kernel: one thread needs ~60 cycles per tcgen05.mma (descriptor
     // arithmetic on the uniform datapath + the elect loop the compiler wraps around UTCHMMA), more than the 48 tensor
     // cycles an N = 96 MMA takes (measured: with the epilogue and the TMA loads switched off the N = 96 layers ran at
-    // 770 TFLOP/s with one issuing thread and 990 with two).  With p.issuers == 2 the two 128-row sub-tiles of a tile
-    // are issued by two warps (sub 0: warp 1, sub 1: warp 10); each commits its own MMAs, so the stage / accumulator
+    // 770 TFLOP/s with one issuing thread and 990 with two).  With MSUB == 2 the two 128-row sub-tiles of a tile
+    // are issued by two warps (sub 0: warp 1, sub 1: warp 18); each commits its own MMAs, so the stage / accumulator
     // barriers expect two arrivals.  The sub-tile range and the tap count are compile-time in mma_role.
     constexpr uint32_t idesc = make_idesc(128 * CG, N);
     if constexpr (GEO == 1) {
@@ -565,7 +537,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
       using J1 = std::integral_constant<int, 1>;
       using JM = std::integral_constant<int, MSUB>;
       using JL = std::integral_constant<int, MSUB - 1>;
-      if (p.issuers == 2) {
+      if constexpr (MSUB == 2) {
         if (warp == 1) run1(J0{}, J1{});
         else run1(JL{}, JM{});
       } else {
@@ -578,25 +550,18 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
     auto run = [&](auto sub_lo_c, auto sub_hi_c) {
       constexpr int SUB_LO = decltype(sub_lo_c)::value, SUB_HI = decltype(sub_hi_c)::value;
       uint32_t stage = 0, phase = 0, acc = 0, acc_phase = 0;
-      const bool prof = TCS_KERNEL_PROFILE && (p.debug & 128) && blockIdx.x == 0 && warp == 1;
-      long long w_empty = 0, w_full = 0, t_begin = prof ? clock64() : 0;
-      int ntile = 0;
       const int stages_per_cb = p.KYG * p.KW;
       for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-        long long c0 = prof ? clock64() : 0;
         ptx::mbar_wait(ptx::smem_u32(&bars.tmem_empty[acc]), acc_phase ^ 1);
         ptx::tc_fence_after();
-        if (prof) { w_empty += clock64() - c0; ++ntile; }
         int ks = 0;
         for (int src = 0; src < p.nsrc; ++src)
           for (int cb = 0; cb < p.cblk[src]; ++cb) {
             // K steps (16 channels each) of this channel block: 4, or 2 for the half block that ends a 96-channel source
             const int ksteps = (cb == p.cblk[src] - 1 && p.ctail[src]) ? 2 : 4;
             for (int sc = 0; sc < stages_per_cb; ++sc, ++ks) {
-              c0 = prof ? clock64() : 0;
               ptx::mbar_wait(ptx::smem_u32(&bars.full[stage]), phase);
               ptx::tc_fence_after();
-              if (prof) w_full += clock64() - c0;
               if (lane == 0) {
                 // descriptors: one base per operand and stage, then 16-byte-unit increments
                 const uint32_t a_base = smem_base + stage * p.stage_bytes;
@@ -645,15 +610,12 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
           }
         if (++acc == 2) { acc = 0; acc_phase ^= 1; }
       }
-      if (prof && lane == 0)
-        printf("[mma N=%d EPI=%d K=%d] tiles %d  cycles/tile %lld  wait tmem_empty %lld  wait full %lld\n", N, EPI, p.kstages, ntile,
-               (clock64() - t_begin) / (ntile ? ntile : 1), w_empty / (ntile ? ntile : 1), w_full / (ntile ? ntile : 1));
     };
     using I0 = std::integral_constant<int, 0>;
     using I1 = std::integral_constant<int, 1>;
     using IM = std::integral_constant<int, MSUB>;
     using IL = std::integral_constant<int, MSUB - 1>;
-    if (p.issuers == 2) {
+    if constexpr (MSUB == 2) {
       if (warp == 1) run(I0{}, I1{});
       else run(IL{}, IM{});
     } else {
@@ -723,15 +685,13 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
             ptx::mbar_wait_sleep(ptx::smem_u32(&bars.fullL[sl]), pl);         // (polls with a back-off: these warps have slack,
             ptx::mbar_wait_sleep(ptx::smem_u32(&bars.emptyA[sa]), pa ^ 1);    //  the issue slots belong to the epilogue warps)
             const uint32_t lbase = l_ring + sl * p.l_bytes, abase = smem_base + sa * p.a_bytes;
-            if (!(p.debug & 64)) {   // (debug bit 64, timing experiments only: windows left stale)
-              // thread = (16-byte channel chunk, cell slot): 8 chunks x 16 slots, or 4 chunks x 32 slots for a half block
-              const uint32_t k = tail ? (t128 & 3) : (t128 & 7);
-              const int slot = tail ? (t128 >> 2) : (t128 >> 3), nslot = tail ? 32 : 16;
-              for (int ci = slot; ci < 9 * CW; ci += nslot) {
-                const int cm = ci / CW, cn = ci - cm * CW;
-                const bool ey = cm == edge_r0 || cm == edge_r1, ex = cn == edge_c0 || cn == edge_c1;
-                blend_cell(lbase, abase, k, cm, cn, ey ? 0.f : 0.25f, ey ? 1.f : 0.75f, ex ? 0.f : 0.25f, ex ? 1.f : 0.75f);
-              }
+            // thread = (16-byte channel chunk, cell slot): 8 chunks x 16 slots, or 4 chunks x 32 slots for a half block
+            const uint32_t k = tail ? (t128 & 3) : (t128 & 7);
+            const int slot = tail ? (t128 >> 2) : (t128 >> 3), nslot = tail ? 32 : 16;
+            for (int ci = slot; ci < 9 * CW; ci += nslot) {
+              const int cm = ci / CW, cn = ci - cm * CW;
+              const bool ey = cm == edge_r0 || cm == edge_r1, ex = cn == edge_c0 || cn == edge_c1;
+              blend_cell(lbase, abase, k, cm, cn, ey ? 0.f : 0.25f, ey ? 1.f : 0.75f, ex ? 0.f : 0.25f, ex ? 1.f : 0.75f);
             }
             ptx::fence_proxy_async();
             __syncwarp();
@@ -746,7 +706,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
     }
   } else if (warp >= 2 && warp < 2 + EPI_WARPS) {
     // ============================== epilogue (2 groups x 8 warps) ================
-    // What the clock64 profile (TCS_DEBUG=128) showed: the epilogue of a tile is a chain of latencies (TMEM loads of
+    // What a clock64 profile showed: the epilogue of a tile is a chain of latencies (TMEM loads of
     // ~1k cycles each while the MMAs run, the GroupNorm exchange between the CTAs of an image, MUFU, proxy fence + TMA
     // stores: ~12k cycles on a K = 864 layer), not of instruction issue, and it does not shrink when the tile is spread
     // over more warps.  So two tiles are kept in flight: group g = 0/1 owns TMEM accumulator set g and therefore every
@@ -788,11 +748,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
         x_ = rem_ - y_ * p.W;
       }
     };
-    uint32_t it = 0;
-    const bool prof = TCS_KERNEL_PROFILE && (p.debug & 128) && blockIdx.x == 0 && e == 0;
-    long long pw_full = 0, p_ld = 0, p_a = 0, p_b = 0, p_c = 0, pc0 = 0, pc1 = 0, q_post = 0, q_poll = 0, q_npoll = 0, r_math = 0;
-    (void)p_ld;
-    long long tacc[3] = {0, 0, 0};
     auto release_tmem = [&]() {
       ptx::tc_fence_before();
       __syncwarp();
@@ -801,16 +756,13 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
         else ptx::mbar_arrive(ptx::smem_u32(&bars.tmem_empty[acc]));
       }
     };
-    for (int tile = blockIdx.x + grp * gridDim.x; tile < n_tiles; tile += 2 * gridDim.x, acc_phase ^= 1, ++it) {
+    for (int tile = blockIdx.x + grp * gridDim.x; tile < n_tiles; tile += 2 * gridDim.x, acc_phase ^= 1) {
       int mt, nt;
       tile_to_mn<CG>(tile, p.n_ntiles, mt, nt);
       const uint32_t tbase = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc * ACC_STRIDE;
       const uint32_t taddr = tbase + h * UC;
-      if (prof) { pc1 = clock64(); if (it) p_c += pc1 - pc0; pc0 = pc1; }
       ptx::mbar_wait(ptx::smem_u32(&bars.tmem_full[acc]), acc_phase);
       ptx::tc_fence_after();
-      if (prof) { pc1 = clock64(); pw_full += pc1 - pc0; pc0 = pc1; }
-      if (p.debug & 16) { release_tmem(); continue; }   // experiment: no epilogue work at all
 
       if constexpr (EPI == EPI_EPS) {
         // ---- 96 -> 1 output conv: column 0 of each sub-tile's accumulator is eps; CFG combine in registers
@@ -869,26 +821,13 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
         float rv[2 * NGL];                     // (sum, sum of squares) per local group
         // Pass 1 reads the accumulator ONCE (32 columns at a time, next tcgen05.ld in flight): statistics in fp32, and the
         // biased values (bias_s holds bias - K_g, see its load) are kept as fp16 (3 more mantissa bits than the bf16 output,
-        // satfinite): column blocks 0 and 1 in
-        // this warp's two output staging blocks (same [32 px][64 B] swizzled rows as the bf16 output that replaces them in
-        // place in pass 2; a lane only ever touches its own row), block 2 in 16 registers.  The TMEM set therefore goes
-        // back to the MMA warps BEFORE the cross-CTA exchange (the accumulator hold time was the bound of the K = 864
-        // layers: ~10k cycles against ~6k of MMA work per tile).
+        // satfinite): column blocks 0 and 1 in the 64 TMEM columns an accumulator set leaves free (192 of 256), 32 per
+        // warp unit, block 2 in 16 registers.  (tcgen05.st / ld do not touch shared memory, whose bandwidth the MMA
+        // operand reads of an N = 96 layer already use to ~90 %.)  The accumulator columns therefore go back to the MMA
+        // warps BEFORE the cross-CTA exchange (the accumulator hold time was the bound of the K = 864 layers: ~10k cycles
+        // against ~6k of MMA work per tile).
         uint32_t stash2[BLK / 2];
-        const uint32_t srow = slab + lane * 64;        // this lane's row inside a staging block
-        const int ssw = (lane >> 1) & 3;
-        const uint32_t sb0 = slab_buf;                 // staging block that pass 2 fills first
-        // TCS_STASH_TMEM (default): column blocks 0 and 1 of the stash live in the 64 TMEM columns an accumulator set
-        // leaves free (192 of 256), 32 per warp unit, instead of the staging blocks: tcgen05.st / ld do not touch shared
-        // memory, whose bandwidth the MMA operand reads of an N = 96 layer already use to ~90 %
-        const bool stash_tmem = !(p.debug & 32);
         const uint32_t tstash = tbase + N * MSUB + h * 32;
-        if (use_tma_out && !stash_tmem) {              // the previous tile's TMA stores have left the staging blocks
-          const long long cl0 = prof ? clock64() : 0;
-          if (lane == 0) ptx::bulk_wait_read<0>();
-          __syncwarp();
-          if (prof) p_ld += clock64() - cl0;
-        }
         {
           float gs[NGL], gq[NGL];
 #pragma unroll
@@ -901,7 +840,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
             if (k < 2) ptx::tmem_ld32(taddr + (k + 1) * 32, vbuf[(k + 1) & 1]);
             else release_tmem();
             const float* v = vbuf[k & 1];
-            const uint32_t sblk = srow + ((sb0 ^ (k & 1)) * 2048);
 #pragma unroll
             for (int i = 0; i < 32; i += 8) {
               uint32_t hw[4];
@@ -919,16 +857,12 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
                 hw[u / 2] = pack_f16x2_sat(t0, t1);
                 hw[u / 2 + 1] = pack_f16x2_sat(t2, t3);
               }
-              if (k < 2 && !stash_tmem) {
-                st_shared_u4(sblk + (((i / 8) ^ ssw) << 4), hw[0], hw[1], hw[2], hw[3]);
-              } else {
 #pragma unroll
-                for (int u = 0; u < 4; ++u) stash2[i / 2 + u] = hw[u];
-              }
+              for (int u = 0; u < 4; ++u) stash2[i / 2 + u] = hw[u];
             }
-            if (k < 2 && stash_tmem) ptx::tmem_st16(tstash + k * 16, stash2);
+            if (k < 2) ptx::tmem_st16(tstash + k * 16, stash2);
           }
-          if (stash_tmem) ptx::tmem_st_wait();
+          ptx::tmem_st_wait();
           // fp16 stash range guard, for free: a row whose sum of squares over a group stays below 65504^2 cannot hold a
           // value that saturated in cvt.rn.satfinite.  Otherwise flag the launch: the host re-runs the evaluation on the
           // unfused path (conv -> fp32 -> GroupNorm kernel) instead of returning a clipped activation.
@@ -959,7 +893,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
         __syncwarp();
         if ((lane & ((32 >> SC_STEPS) - 1)) == 0) gsm->red[ew][2 * (col0 / CPGN) + idx] = rv[0];
         epi_bar_sync(grp);
-        if (prof) { pc1 = clock64(); p_a += pc1 - pc0; pc0 = pc1; }
         if (ew == 0) {
           // Exchange between the G CTAs of the image, one L2 round trip each way: every (value, flag) pair is ONE 64-bit
           // word (the flag travels with the data, as in NCCL's LL protocol), so there is no separate counter, no fence and
@@ -971,13 +904,11 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
             for (int w = 0; w < GRP_WARPS; ++w) tot += gsm->red[w][lane];
             st_relaxed_gpu_u64(ll + static_cast<size_t>(mt) * 16 + lane, (1ULL << 32) | __float_as_uint(tot));
           }
-          if (prof) { pc1 = clock64(); q_post += pc1 - pc0; }
           // 16 values x G CTAs: lane l sums value (l & 15) over the CTAs of parity (l >> 4), fixed order
           const unsigned long long* ip = ll + static_cast<size_t>(img) * G * 16 + (lane & 15);
           float part = 0.f;
           {
             const long long t0 = clock64();
-            int polls = 0;
             unsigned long long w[8];        // G <= 16: at most 8 words per lane, all loads in flight together
             bool ready;
             do {
@@ -989,15 +920,10 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
               }
 #pragma unroll
               for (int i = 0; i < 8; ++i) ready = ready && ((w[i] >> 32) == 1ULL);
-              if (p.debug & 1) ready = true;
-              if (!ready) {
-                ++polls;
-                if (clock64() - t0 > p.exch_timeout) __trap();   // -> launch failure, reported as TCS_ERR_CUDA
-              }
+              if (!ready && clock64() - t0 > EXCHANGE_TIMEOUT_CYCLES) __trap();   // -> launch failure, reported as TCS_ERR_CUDA
             } while (!ready);
 #pragma unroll
             for (int i = 0; i < 8; ++i) part += __uint_as_float(static_cast<uint32_t>(w[i]));   // zeros for k >= G
-            if (prof) { q_poll += clock64() - pc1; q_npoll += polls; }
           }
           part += __shfl_xor_sync(0xffffffffu, part, 16);
           const float qsum = __shfl_down_sync(0xffffffffu, part, 1);   // lane 2g: sum, lane 2g+1: sum of squares
@@ -1019,7 +945,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
           }
         }
         epi_bar_sync(grp);
-        if (prof) { pc1 = clock64(); p_b += pc1 - pc0; pc0 = pc1; }
         __nv_bfloat16* obase = static_cast<__nv_bfloat16*>(p.epi.out);
         int img_px, y, x;
         pixel_of(mt, img_px, y, x);
@@ -1031,13 +956,9 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
         for (int k = 0; k < 3; ++k) {
           const int cc = col0 + k * 32;
           uint32_t hv[16];
-          if (k < 2 && stash_tmem) {
+          if (k < 2) {
             ptx::tmem_ld16(tstash + k * 16, reinterpret_cast<float*>(hv));
             ptx::tmem_ld_wait();
-          } else if (k < 2) {
-            const uint32_t sblk = srow + ((sb0 ^ k) * 2048);   // = the block store_padded_block fills next (in place)
-#pragma unroll
-            for (int j = 0; j < 4; ++j) ld_shared_u4(sblk + ((j ^ ssw) << 4), hv[4 * j], hv[4 * j + 1], hv[4 * j + 2], hv[4 * j + 3]);
           } else {
 #pragma unroll
             for (int j = 0; j < 16; ++j) hv[j] = stash2[j];
@@ -1056,12 +977,9 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
             pk[i / 2] = pack_bf16x2(y0, y1);
             pk[i / 2 + 1] = pack_bf16x2(y2, y3);
           }
-          if (!(p.debug & 2))
-            store_padded_block<GEO>(&mapO, use_tma_out, slab, slab_buf, lane, obase, pix, wy, wx, Wp, p.epi.ldo, cc, img, y, x, pk,
-                                    prof ? tacc : nullptr, GEO == 1 ? 0 : h16, &mapO1, p.H);
-          else if (pk[0] == 0x12345678u && pk[7] == 0x9abcdef0u) obase[0] = __float2bfloat16(0.f);
+          store_padded_block<GEO>(&mapO, use_tma_out, slab, slab_buf, lane, obase, pix, wy, wx, Wp, p.epi.ldo, cc, img, y, x, pk,
+                                  GEO == 1 ? 0 : h16, &mapO1, p.H);
         }
-        if (prof) r_math += clock64() - pc1;
       } else if constexpr (N >= 96) {
         const int n_off = nt * N + col0;                     // first output channel of this warp's columns
         int b, y, x;
@@ -1071,7 +989,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
         ptx::tmem_ld32(taddr, vbuf[0]);
         if constexpr (EPI == EPI_RAW_STATS) {
           // fp32 output (one row per lane, plain stores) plus per-(warp, group) partial sums for a separate GroupNorm
-          // pass: the unfused A/B path (TCS_FUSE_GN=0) and the per-layer tests; not on the production path
+          // pass: the unfused path (fuse_gn off, or the re-run after an fp16 stash overflow) and the per-layer tests; not
+          // on the production path
           constexpr int CPGN = N / 8;
           constexpr int NG = UC / CPGN;
           float gs[NG], gq[NG];
@@ -1147,7 +1066,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
               pk[i / 2 + 1] = pack_bf16x2(v[i + 2] + b4.z, v[i + 3] + b4.w);
             }
             store_padded_block<GEO, SB>(&mapO, use_tma_out, slab, slab_buf, lane, obase, pix, wy, wx, Wp, p.epi.ldo, n_off + c0, b, y, x, pk,
-                                        nullptr, GEO == 1 ? 0 : h16, &mapO1, p.H);
+                                        GEO == 1 ? 0 : h16, &mapO1, p.H);
           }
         } else {  // EPI_PLAIN: unpadded bf16 [pixel][ldo] rows; 32 px x 32 ch blocks staged in the warp's slabs and
                   // TMA-stored (a lane-per-row 16-byte store touches 32 different lines per instruction)
@@ -1190,9 +1109,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
         }
       }
     }
-    if (prof && lane == 0 && it > 1)
-      printf("[epi N=%d EPI=%d] per tile: wait tmem_full %lld  staging-block wait %lld  pass1+barA %lld  exchange+table+barB %lld (post %lld, poll %lld, polls %lld)  pass2+stores+loop %lld (pass2 %lld: wait_read %lld, sts+fence %lld, tma issue %lld)\n",
-             N, EPI, pw_full / it, p_ld / it, p_a / it, p_b / it, q_post / it, q_poll / it, q_npoll / it, p_c / (it - 1), r_math / it, tacc[0] / it, tacc[1] / it, tacc[2] / it);
     if (lane == 0) ptx::bulk_wait_all();   // staged TMA stores have left shared memory
   }
 
@@ -1240,8 +1156,7 @@ void conv_tc_tile_shape(const ConvGeom& g, int epi, int* N, int* cg) {
   if (*N >= 96 && g.ksize >= 3) *cg = 2;
   // the 96 -> 1 output conv is bound by MMA ISSUE (36 tiny N = 16 MMAs per tile at ~100 cycles each): as a CTA pair one
   // thread's MMA covers both CTAs' tiles, which halves the issue work per tile
-  const char* e2 = getenv("TCS_EPS_CG");
-  if (epi == EPI_EPS && !(e && atoi(e) == 1) && !(e2 && atoi(e2) == 1)) *cg = 2;
+  if (epi == EPI_EPS && !(e && atoi(e) == 1)) *cg = 2;
 }
 
 // Packed layout: [K stage][N tile][CTA of the pair][tap][N/cg rows][64 channels], every 128-byte row with its 16-byte
@@ -1338,9 +1253,8 @@ int conv_tc_grid(const ConvTcPlan& pl, int B, int sm_count) {
   // at most one grid-stride ahead, whose CTAs never wait for anything later).  Whole image groups (grid a multiple of the
   // tiles per image) keep every image inside one wave; the full grid lets one image in ~9 straddle two waves (its first
   // tiles' epilogue group waits one tile period, which the other group and the double-buffered accumulators absorb) but
-  // uses all SMs: 148 instead of 144 on the 64x64 and 32x32 layers.  TCS_GN_GROUP_GRID=1 restores the rounded grid.
-  static const bool group_grid = getenv("TCS_GN_GROUP_GRID") && atoi(getenv("TCS_GN_GROUP_GRID")) == 1;
-  if (pl.epi == EPI_GN_FUSED && (group_grid || grid < pl.p.tiles_per_img * 2))
+  // uses all SMs: 148 instead of 144 on the 64x64 and 32x32 layers.  A grid of fewer than two image groups is rounded.
+  if (pl.epi == EPI_GN_FUSED && grid < pl.p.tiles_per_img * 2)
     grid = grid / pl.p.tiles_per_img * pl.p.tiles_per_img;
   if (pl.cg == 2) grid &= ~1;                                                         // whole CTA pairs
   return grid;
@@ -1364,7 +1278,6 @@ static bool coop_cluster_supported() {
     const cudaError_t e = cudaLaunchKernelEx(&cfg, coop_cluster_probe_kernel);
     cudaGetLastError();
     state = (e == cudaSuccess && cudaDeviceSynchronize() == cudaSuccess) ? 1 : 0;
-    if (getenv("TCS_NO_COOP_CLUSTER")) state = 0;
   }
   return state == 1;
 }
@@ -1524,11 +1437,6 @@ int conv_tc_make_plan(ConvTcPlan* plan, const ConvGeom& g, const void* src0, con
   if (g.H % (pl.msub * (128 / g.W))) return fail(TCS_ERR_UNSUPPORTED, "conv_tc: image height not a multiple of the tile");
   p.debug = getenv("TCS_DEBUG") ? atoi(getenv("TCS_DEBUG")) : 0;
   p.gn_inv_cnt = 1.0 / (static_cast<double>(g.H) * g.W * (pl.N / 8));
-  p.exch_timeout = getenv("TCS_EXCHANGE_TIMEOUT") ? atoll(getenv("TCS_EXCHANGE_TIMEOUT")) : EXCHANGE_TIMEOUT_CYCLES;
-  {
-    const char* e = getenv("TCS_ISSUERS");   // 1 = a single MMA-issuing thread everywhere (A/B switch)
-    p.issuers = (pl.msub == 2 && !(e && atoi(e) == 1)) ? 2 : 1;
-  }
   stage_shape(g, &p.T, &p.KYG, &p.KW);
   p.H = g.H; p.W = g.W; p.Rt = 128 / g.W;
   p.stride = g.stride;
@@ -1584,8 +1492,7 @@ int conv_tc_make_plan(ConvTcPlan* plan, const ConvGeom& g, const void* src0, con
     // what to do with the 32 KB (measured, profiles/r2_layer_speed_fused_upsample.txt): us1_conv (N = 96, a 64- and a
     // 32-channel block per tile) gains 2 % from a third window stage (2 weight stages left), us2_conv (N = 192) gains 5 %
     // from a third weight stage instead
-    const bool want3 = getenv("TCS_UPS_A_STAGES") ? atoi(getenv("TCS_UPS_A_STAGES")) == 3 : pl.msub == 2;
-    if (g.ups && want3 && budget1 >= 3 * static_cast<size_t>(p.a_bytes) + 2 * static_cast<size_t>(3u * NB * ROWB))
+    if (g.ups && pl.msub == 2 && budget1 >= 3 * static_cast<size_t>(p.a_bytes) + 2 * static_cast<size_t>(3u * NB * ROWB))
       p.a_stages = 3;
     const size_t rest = budget1 - static_cast<size_t>(p.a_stages) * p.a_bytes;
     p.tb = (rest / (3u * NB * ROWB) >= (g.ups ? 2u : 3u)) ? 3 : 1;   // (ups: two 3-tap stages beat seven 1-tap stages)
@@ -1593,8 +1500,6 @@ int conv_tc_make_plan(ConvTcPlan* plan, const ConvGeom& g, const void* src0, con
     p.stage_bytes = (static_cast<uint32_t>(p.tb) * NB * ROWB + 1023u) & ~1023u;
     p.nstage = static_cast<int>(rest / p.stage_bytes);
     if (p.nstage > MAX_STAGES) p.nstage = MAX_STAGES;
-    if (getenv("TCS_NSTAGE") && atoi(getenv("TCS_NSTAGE")) < p.nstage) p.nstage = atoi(getenv("TCS_NSTAGE"));   // experiment
-    if (getenv("TCS_PLAN_LOG")) fprintf(stderr, "[conv_tc plan] H=%d N=%d K=%d ups=%d tb=%d nstage=%d stage_bytes=%u a_bytes=%u l_bytes=%u\n", g.H, pl.N, p.kstages, p.ups, p.tb, p.nstage, p.stage_bytes, p.a_bytes, p.l_bytes);
     if (p.nstage < 2) return fail(TCS_ERR_UNSUPPORTED, "conv_tc: weight stage does not fit shared memory twice");
     pl.smem = static_cast<size_t>(p.a_stages) * p.a_bytes + static_cast<size_t>(p.l_stages) * p.l_bytes +
               static_cast<size_t>(p.nstage) * p.stage_bytes + 1024 + slab_bytes + bias_bytes_of(g.ntot) + EPI_FUSED_BYTES;

@@ -25,8 +25,6 @@ struct ConvTcParams {
   int kxn;                  // EPI_EPS: 1 = kx taps live in accumulator columns 0..2 (ConvGeom::kx_in_n)
   float guidance;           // EPI_EPS with pair: eps = e_u + guidance (e_c - e_u)
   double gn_inv_cnt;        // EPI_GN_FUSED: 1 / (H * W * channels per group)
-  long long exch_timeout;   // EPI_GN_FUSED: cycles a CTA waits for its image group's partial sums before it traps
-  int issuers;              // MMA-issuing warps: 2 = one per 128-row sub-tile (MSUB == 2), 1 otherwise
   // geo = 1 ("tap-shift" geometry, 3x3 stride-1 layers): a 128-row sub-tile is 16 image rows x 8 pixels, the A operand
   // of a 64-channel block is ONE (16 + 2) x (8 MSUB + 2) pixel window in its own ring, and the nine taps are descriptor
   // start shifts into it; the weights stream through a second ring in stages of `tb` taps
@@ -38,7 +36,7 @@ struct ConvTcParams {
   int ups;                  // 1 = fused bilinear x2 upsample (ConvGeom::ups): low-resolution windows in a ring of l_stages slots
   int l_stages;
   uint32_t l_bytes, l_load_bytes;
-  int debug;                // TCS_DEBUG bits (timing experiments only): 1 = no inter-CTA wait, 2 = no pass-2 stores
+  int debug;                // TCS_DEBUG bits: 4 = per-lane stores instead of TMA stores (the reference of the TMA epilogues)
   EpiArgs epi;
 };
 

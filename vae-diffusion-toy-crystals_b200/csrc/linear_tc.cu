@@ -24,8 +24,6 @@
 // zero fill TMA applies outside the tensor IS the transposed convolution's implicit zero border.
 #include "linear_tc.cuh"
 
-#include <cstdlib>
-
 #include "tc_ptx.cuh"
 
 namespace tcs {
@@ -56,24 +54,19 @@ __device__ __forceinline__ uint32_t lt_pack(float a, float b) {
   return *reinterpret_cast<const uint32_t*>(&h);
 }
 
-// tile -> (M tile, N tile [for CONV: N tile index = parity class, the weight matrices of the 4 classes are stacked])
-template <int CG>
+// tile -> (M tile, N tile [for CONV: N tile index = parity class, the weight matrices of the 4 classes are stacked]);
+// the two CTAs of a pair (consecutive tile indices) share the N tile
 __device__ __forceinline__ void lt_tile_to_mn(int tile, int n_mtiles, int& mt, int& nt) {
-  if (CG == 2) {   // the two CTAs of a pair (consecutive tile indices) share the N tile
-    const int pt = tile >> 1, half = n_mtiles >> 1;
-    nt = pt / half;
-    mt = ((pt - nt * half) << 1) | (tile & 1);
-  } else {
-    nt = tile / n_mtiles;
-    mt = tile - nt * n_mtiles;
-  }
+  const int pt = tile >> 1, half = n_mtiles >> 1;
+  nt = pt / half;
+  mt = ((pt - nt * half) << 1) | (tile & 1);
 }
 // transposed-conv tap (ty, tx) of parity (py, px): input offset per axis
 __device__ __forceinline__ int lt_tap_off(int parity_bit, int tap_bit) {
   return parity_bit == 0 ? (tap_bit == 0 ? 0 : -1) : (tap_bit == 0 ? 1 : 0);
 }
 
-template <int CG, int BN, bool CONV>
+template <int BN, bool CONV>
 __global__ void __launch_bounds__(LT_THREADS, 1)
 linear_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapW,
                  const __grid_constant__ CUtensorMap mapO, const LinearTcParams p) {
@@ -84,7 +77,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0), lane = threadIdx.x & 31;   // warp-uniform for the compiler
   const uint32_t smem_base = (ptx::smem_u32(smem_raw) + 1023u) & ~1023u;
   const int n_tiles = p.n_mtiles * p.n_ntiles;
-  constexpr int NB = LT_BN / CG;                 // W rows this CTA stages per K block
+  constexpr int NB = LT_BN / 2;                  // W rows this CTA stages per K block
   constexpr uint32_t B_BYTES = NB * LT_BK * 2;
 
   if (warp == 0 && lane == 0) {
@@ -97,18 +90,15 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
     }
     for (int a = 0; a < 2; ++a) {
       ptx::mbar_init(ptx::smem_u32(&bars.tmem_full[a]), 1);
-      ptx::mbar_init(ptx::smem_u32(&bars.tmem_empty[a]), LT_EPI_WARPS * CG);
+      ptx::mbar_init(ptx::smem_u32(&bars.tmem_empty[a]), LT_EPI_WARPS * 2);
     }
     ptx::fence_barrier_init();
   }
-  const uint32_t cta_rank = (CG == 2) ? ptx::cluster_ctarank() : 0u;
-  if (warp == 1) {
-    if (CG == 2) ptx::tmem_alloc_512_2sm(ptx::smem_u32(&bars.tmem_base));
-    else ptx::tmem_alloc_512(ptx::smem_u32(&bars.tmem_base));
-  }
+  const uint32_t cta_rank = ptx::cluster_ctarank();
+  if (warp == 1) ptx::tmem_alloc_512_2sm(ptx::smem_u32(&bars.tmem_base));
   ptx::tc_fence_before();
   __syncthreads();
-  if (CG == 2) ptx::cluster_sync_all();
+  ptx::cluster_sync_all();
   ptx::tc_fence_after();
   const uint32_t tmem_base = bars.tmem_base;
 
@@ -117,7 +107,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
     uint32_t stage = 0, phase = 0;
     for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
       int mt, nt;
-      lt_tile_to_mn<CG>(tile, p.n_mtiles, mt, nt);
+      lt_tile_to_mn(tile, p.n_mtiles, mt, nt);
       // CONV: the 128 rows of an M tile are `imgs` whole images (Hi*Hi < 128) or `rows_y` rows of one image
       int b0 = 0, y0 = 0;
       if (CONV) {
@@ -126,37 +116,27 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
       }
       for (int kb = 0; kb < p.kblocks; ++kb) {
         ptx::mbar_wait(ptx::smem_u32(&bars.empty[stage]), phase ^ 1);
-        if ((p.debug & 2) && (phase || tile != static_cast<int>(blockIdx.x))) {   // experiment: operands stay stale
-          if (lane == 0 && (CG == 1 || cta_rank == 0)) ptx::mbar_arrive(ptx::smem_u32(&bars.full[stage]));
-          __syncwarp();
-          if (++stage == static_cast<uint32_t>(p.nstage)) { stage = 0; phase ^= 1; }
-          continue;
-        }
         if (lane == 0) {
           const uint32_t full = ptx::smem_u32(&bars.full[stage]);
           const uint32_t a_dst = smem_base + stage * p.stage_bytes;
           const uint32_t b_dst = a_dst + p.a_bytes;
-          if (CG == 2 && cta_rank == 0) ptx::mbar_expect_tx(full, 2 * (p.a_bytes + B_BYTES));
-          if (CG == 1) ptx::mbar_expect_tx(full, p.a_bytes + B_BYTES);
+          if (cta_rank == 0) ptx::mbar_expect_tx(full, 2 * (p.a_bytes + B_BYTES));
           if (CONV) {
             const int tap = kb / p.cblocks, cb = kb - tap * p.cblocks;
             const int dy = lt_tap_off(nt >> 1, tap >> 1), dx = lt_tap_off(nt & 1, tap & 1);
-            if (CG == 2) ptx::tma_load_4d_2sm(a_dst, &mapA, full, cb * LT_BK, dx, y0 + dy, b0);
-            else ptx::tma_load_4d(a_dst, &mapA, full, cb * LT_BK, dx, y0 + dy, b0);
+            ptx::tma_load_4d_2sm(a_dst, &mapA, full, cb * LT_BK, dx, y0 + dy, b0);
           } else {
-            if (CG == 2) ptx::tma_load_2d_2sm(a_dst, &mapA, full, kb * LT_BK, mt * LT_BM);
-            else ptx::tma_load_2d(a_dst, &mapA, full, kb * LT_BK, mt * LT_BM);
+            ptx::tma_load_2d_2sm(a_dst, &mapA, full, kb * LT_BK, mt * LT_BM);
           }
-          if (CG == 2) ptx::tma_load_2d_2sm(b_dst, &mapW, full, kb * LT_BK, nt * LT_BN + static_cast<int>(cta_rank) * NB);
-          else ptx::tma_load_2d(b_dst, &mapW, full, kb * LT_BK, nt * LT_BN);
+          ptx::tma_load_2d_2sm(b_dst, &mapW, full, kb * LT_BK, nt * LT_BN + static_cast<int>(cta_rank) * NB);
         }
         __syncwarp();
         if (++stage == static_cast<uint32_t>(p.nstage)) { stage = 0; phase ^= 1; }
       }
     }
   } else if (warp == 1 && cta_rank == 0) {
-    // ============================== MMA issuer (leader CTA only when CG == 2) ====
-    constexpr uint32_t idesc = make_idesc(LT_BM * CG, LT_BN);
+    // ============================== MMA issuer (leader CTA only) =================
+    constexpr uint32_t idesc = make_idesc(LT_BM * 2, LT_BN);
     uint32_t stage = 0, phase = 0, acc = 0, acc_phase = 0;
     for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
       ptx::mbar_wait(ptx::smem_u32(&bars.tmem_empty[acc]), acc_phase ^ 1);
@@ -171,16 +151,10 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
 #pragma unroll
           for (int k = 0; k < LT_BK / 16; ++k) {   // 32 bytes per K = 16 step inside the 128-byte swizzle row
             const uint32_t accum = (kb | k) != 0 ? 1u : 0u;
-            if (CG == 2) ptx::umma_bf16_2sm(d_tmem, adesc + k * 2, bdesc + k * 2, idesc, accum);
-            else ptx::umma_bf16(d_tmem, adesc + k * 2, bdesc + k * 2, idesc, accum);
+            ptx::umma_bf16_2sm(d_tmem, adesc + k * 2, bdesc + k * 2, idesc, accum);
           }
-          if (CG == 2) {
-            ptx::umma_commit_2sm(ptx::smem_u32(&bars.empty[stage]));
-            if (kb == p.kblocks - 1) ptx::umma_commit_2sm(ptx::smem_u32(&bars.tmem_full[acc]));
-          } else {
-            ptx::umma_commit(ptx::smem_u32(&bars.empty[stage]));
-            if (kb == p.kblocks - 1) ptx::umma_commit(ptx::smem_u32(&bars.tmem_full[acc]));
-          }
+          ptx::umma_commit_2sm(ptx::smem_u32(&bars.empty[stage]));
+          if (kb == p.kblocks - 1) ptx::umma_commit_2sm(ptx::smem_u32(&bars.tmem_full[acc]));
         }
         __syncwarp();
         if (++stage == static_cast<uint32_t>(p.nstage)) { stage = 0; phase ^= 1; }
@@ -203,7 +177,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
     const bool silu = (p.flags & LIN_SILU) != 0, f32 = (p.flags & LIN_OUT_F32) != 0, accum = (p.flags & LIN_ACCUM) != 0;
     for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
       int mt, nt;
-      lt_tile_to_mn<CG>(tile, p.n_mtiles, mt, nt);
+      lt_tile_to_mn(tile, p.n_mtiles, mt, nt);
       const int r = q * 32 + lane;
       size_t row = static_cast<size_t>(mt) * LT_BM + r;     // output row (pixel) index
       bool live = row < static_cast<size_t>(p.M);
@@ -226,7 +200,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
       const uint32_t tbase = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc * ACC_COLS;
       // bias of this N tile -> shared memory (while the main loop of the tile is still running)
       float* bs = bias_s + acc * 256;
-      if (et < LT_BN) bs[et] = (p.bias && !(p.debug & 32)) ? __ldg(p.bias + col0 + et) : 0.f;
+      if (et < LT_BN) bs[et] = p.bias ? __ldg(p.bias + col0 + et) : 0.f;
       asm volatile("bar.sync 1, %0;" ::"n"(32 * LT_EPI_WARPS) : "memory");
       ptx::mbar_wait(ptx::smem_u32(&bars.tmem_full[acc]), acc_phase);
       ptx::tc_fence_after();
@@ -240,10 +214,6 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
         if (cc + 1 < CPW) ptx::tmem_ld32(tbase + (c + 1) * 32, vbuf[(cc + 1) & 1]);
         float* v = vbuf[cc & 1];
         const int col = col0 + c * 32;
-        if (p.debug & 1) {   // experiment: no global traffic in the epilogue
-          if (v[0] == 1.2345e-30f && live) static_cast<float*>(p.out)[0] = v[1];
-          continue;
-        }
         {
 #pragma unroll
           for (int i = 0; i < 32; i += 4) {
@@ -251,7 +221,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
             v[i] += b4.x; v[i + 1] += b4.y; v[i + 2] += b4.z; v[i + 3] += b4.w;
           }
         }
-        if (silu && !(p.debug & 16)) {
+        if (silu) {
 #pragma unroll
           for (int i = 0; i < 32; ++i) v[i] = lt_silu(v[i]);
         }
@@ -259,7 +229,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
 #pragma unroll
           for (int i = 0; i < 32; ++i) v[i] = fmaxf(v[i], 0.f);
         }
-        if (!CONV && !(p.debug & 4)) {
+        if (!CONV) {
           // 32 rows x 32 columns -> swizzled slab -> one TMA store / reduce-add per block (full 128-byte lines)
           if (lane == 0) ptx::bulk_wait_read<1>();   // the slab half written two blocks ago has been read
           __syncwarp();
@@ -283,7 +253,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
           __syncwarp();
           if (lane == 0) {
             const int r0 = mt * LT_BM + q * 32;
-            if (r0 < p.M && !(p.debug & 8)) {   // rows past M inside the box are clipped by the tensor map
+            if (r0 < p.M) {   // rows past M inside the box are clipped by the tensor map
               if (accum) ptx::tma_reduce_add_2d(&mapO, base, col, r0);
               else ptx::tma_store_2d(&mapO, base, col, r0);
             }
@@ -311,10 +281,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
       }
       ptx::tc_fence_before();
       __syncwarp();
-      if (lane == 0) {
-        if (CG == 2) ptx::mbar_arrive_rank0(ptx::smem_u32(&bars.tmem_empty[acc]));
-        else ptx::mbar_arrive(ptx::smem_u32(&bars.tmem_empty[acc]));
-      }
+      if (lane == 0) ptx::mbar_arrive_rank0(ptx::smem_u32(&bars.tmem_empty[acc]));
       if (++acc == 2) { acc = 0; acc_phase ^= 1; }
     }
     if (!CONV && lane == 0) ptx::bulk_wait_all();   // staged TMA stores have completed
@@ -322,12 +289,9 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
 
   ptx::tc_fence_before();
   __syncthreads();
-  if (CG == 2) ptx::cluster_sync_all();   // the leader's MMAs read the peer's shared memory / write its TMEM
+  ptx::cluster_sync_all();   // the leader's MMAs read the peer's shared memory / write its TMEM
   ptx::tc_fence_after();
-  if (warp == 1) {
-    if (CG == 2) ptx::tmem_dealloc_512_2sm(tmem_base);
-    else ptx::tmem_dealloc_512(tmem_base);
-  }
+  if (warp == 1) ptx::tmem_dealloc_512_2sm(tmem_base);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -372,34 +336,26 @@ int linear_tc_make_plan(LinearTcPlan* plan, const __nv_bfloat16* A, int lda, con
   if ((flags & LIN_ACCUM) && !(flags & LIN_OUT_F32)) return fail(TCS_ERR_BAD_ARGUMENT, "linear_tc: accumulate needs fp32 output");
   LinearTcPlan& pl = *plan;
   pl = LinearTcPlan();
-  {
-    const char* e = getenv("TCS_CG");   // 1 = single-CTA MMA (A/B switch)
-    pl.cg = (e && atoi(e) == 1) ? 1 : 2;
-  }
   pl.bn = LT_BN;
   pl.conv = false;
   LinearTcParams& p = pl.p;
   p = LinearTcParams();
   p.M = M; p.N = N; p.K = K;
   p.n_mtiles = (M + LT_BM - 1) / LT_BM;
-  if (pl.cg == 2 && (p.n_mtiles & 1)) ++p.n_mtiles;   // whole CTA pairs: the extra tile is all out-of-bounds rows
+  if (p.n_mtiles & 1) ++p.n_mtiles;   // whole CTA pairs: the extra tile is all out-of-bounds rows
   p.n_ntiles = N / LT_BN;
   p.kblocks = K / LT_BK;
   p.a_bytes = LT_BM * LT_BK * 2;
-  p.stage_bytes = p.a_bytes + (LT_BN / pl.cg) * LT_BK * 2;
+  p.stage_bytes = p.a_bytes + (LT_BN / 2) * LT_BK * 2;
   const size_t budget = 227 * 1024 - 2048 - 1024 - LT_SLAB_BYTES - LT_BIAS_BYTES;
   p.nstage = static_cast<int>(budget / p.stage_bytes);
   if (p.nstage > LT_MAX_STAGES) p.nstage = LT_MAX_STAGES;
   pl.smem = static_cast<size_t>(p.nstage) * p.stage_bytes + 1024 + LT_SLAB_BYTES + LT_BIAS_BYTES;
   p.bias = bias; p.out = out; p.ldo = ldo; p.flags = flags;
-  p.debug = getenv("TCS_LT_DEBUG") ? atoi(getenv("TCS_LT_DEBUG")) : 0;
-  if (getenv("TCS_LT_STAGES") && atoi(getenv("TCS_LT_STAGES")) >= 2 && atoi(getenv("TCS_LT_STAGES")) < p.nstage)
-    p.nstage = atoi(getenv("TCS_LT_STAGES"));
   const int tiles = p.n_mtiles * p.n_ntiles;
-  pl.grid = tiles < sm_count ? tiles : sm_count;
-  if (pl.cg == 2) pl.grid &= ~1;
+  pl.grid = (tiles < sm_count ? tiles : sm_count) & ~1;
   TCS_CHECK(lt_encode_2d(&pl.mapA, A, M, K, lda, LT_BM));
-  TCS_CHECK(lt_encode_2d(&pl.mapW, W, N, K, ldw, LT_BN / pl.cg));
+  TCS_CHECK(lt_encode_2d(&pl.mapW, W, N, K, ldw, LT_BN / 2));
   {   // output: 32-column x 32-row boxes, written (bf16 / fp32) or reduce-added (fp32) by TMA from swizzled slabs
     PFN_encodeTiled encode = lt_get_encode();
     const bool f32 = (flags & LIN_OUT_F32) != 0;
@@ -439,7 +395,6 @@ int linear_tc_make_convt_plan(LinearTcPlan* plan, const __nv_bfloat16* in, const
     return fail(TCS_ERR_UNSUPPORTED, "linear_tc convT: needs Hi in {4,8,16}, C_in % 64 == 0, C_out in {32,64,128}");
   LinearTcPlan& pl = *plan;
   pl = LinearTcPlan();
-  pl.cg = 2;
   pl.bn = Co;
   pl.conv = true;
   LinearTcParams& p = pl.p;
@@ -455,7 +410,7 @@ int linear_tc_make_convt_plan(LinearTcPlan* plan, const __nv_bfloat16* in, const
   p.n_ntiles = 4;                     // the parity classes
   p.kblocks = 4 * p.cblocks;
   p.a_bytes = LT_BM * LT_BK * 2;
-  p.stage_bytes = p.a_bytes + (Co / pl.cg) * LT_BK * 2;
+  p.stage_bytes = p.a_bytes + (Co / 2) * LT_BK * 2;
   const size_t budget = 227 * 1024 - 2048 - 1024 - LT_SLAB_BYTES - LT_BIAS_BYTES;
   p.nstage = static_cast<int>(budget / p.stage_bytes);
   if (p.nstage > LT_MAX_STAGES) p.nstage = LT_MAX_STAGES;
@@ -464,15 +419,15 @@ int linear_tc_make_convt_plan(LinearTcPlan* plan, const __nv_bfloat16* in, const
   const int tiles = p.n_mtiles * p.n_ntiles;
   pl.grid = (tiles < sm_count ? tiles : sm_count) & ~1;
   TCS_CHECK(lt_encode_4d(&pl.mapA, in, n, Hi, Ci, p.rows_y, p.imgs));
-  TCS_CHECK(lt_encode_2d(&pl.mapW, wpacked, 4 * Co, 4 * Ci, 4 * Ci, Co / pl.cg));
+  TCS_CHECK(lt_encode_2d(&pl.mapW, wpacked, 4 * Co, 4 * Ci, 4 * Ci, Co / 2));
   pl.mapO = pl.mapW;   // unused: the scattered (stride-2 pixel) rows are stored per lane
   pl.valid = true;
   return TCS_OK;
 }
 
-template <int CG, int BN, bool CONV>
+template <int BN, bool CONV>
 static int lt_launch_t(const LinearTcPlan& pl, cudaStream_t st) {
-  auto kern = linear_tc_kernel<CG, BN, CONV>;
+  auto kern = linear_tc_kernel<BN, CONV>;
   static bool attr_done = false;
   if (!attr_done) {
     TCS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 2048));
@@ -481,13 +436,9 @@ static int lt_launch_t(const LinearTcPlan& pl, cudaStream_t st) {
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(pl.grid); cfg.blockDim = dim3(LT_THREADS); cfg.dynamicSmemBytes = pl.smem; cfg.stream = st;
   cudaLaunchAttribute at[1];
-  int na = 0;
-  if (CG == 2) {
-    at[na].id = cudaLaunchAttributeClusterDimension;
-    at[na].val.clusterDim.x = 2; at[na].val.clusterDim.y = 1; at[na].val.clusterDim.z = 1;
-    ++na;
-  }
-  cfg.attrs = at; cfg.numAttrs = na;
+  at[0].id = cudaLaunchAttributeClusterDimension;
+  at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+  cfg.attrs = at; cfg.numAttrs = 1;
   TCS_CUDA(cudaLaunchKernelEx(&cfg, kern, pl.mapA, pl.mapW, pl.mapO, pl.p));
   TCS_CUDA(cudaGetLastError());
   return TCS_OK;
@@ -496,11 +447,11 @@ static int lt_launch_t(const LinearTcPlan& pl, cudaStream_t st) {
 int linear_tc_launch(const LinearTcPlan& pl, cudaStream_t st) {
   if (!pl.valid) return fail(TCS_ERR_STATE, "linear_tc_launch: plan not built");
   if (pl.conv) {
-    if (pl.bn == 128) return lt_launch_t<2, 128, true>(pl, st);
-    if (pl.bn == 64) return lt_launch_t<2, 64, true>(pl, st);
-    return lt_launch_t<2, 32, true>(pl, st);
+    if (pl.bn == 128) return lt_launch_t<128, true>(pl, st);
+    if (pl.bn == 64) return lt_launch_t<64, true>(pl, st);
+    return lt_launch_t<32, true>(pl, st);
   }
-  return pl.cg == 2 ? lt_launch_t<2, 256, false>(pl, st) : lt_launch_t<1, 256, false>(pl, st);
+  return lt_launch_t<256, false>(pl, st);
 }
 
 }  // namespace tcs

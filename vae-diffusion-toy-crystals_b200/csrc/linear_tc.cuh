@@ -21,7 +21,6 @@ struct LinearTcParams {
   void* out;
   int ldo;                           // elements between output rows
   int flags;
-  int debug;                         // TCS_LT_DEBUG bits (timing experiments only): 1 = epilogue does no global traffic, 2 = no TMA after the first ring fill
   // transposed-convolution mode (linear_tc_make_convt_plan): M tiles are windows of the NHWC input
   int Hi, n_img, cblocks;            // input size, images, 64-channel blocks per tap (kblocks = 4 * cblocks)
   int tiles_per_img, rows_y, imgs;   // M tile = `imgs` whole images (Hi*Hi < 128) or `rows_y` rows of one image
@@ -30,7 +29,6 @@ struct LinearTcParams {
 struct LinearTcPlan {
   CUtensorMap mapA, mapW, mapO;
   LinearTcParams p;
-  int cg;        // 1 = one CTA per MMA, 2 = CTA pairs (cta_group::2, W tile split across the pair)
   int bn;        // N tile: 256 (Linear) or C_out (transposed conv: 128 / 64 / 32)
   bool conv = false;
   int grid;

@@ -141,7 +141,7 @@ using namespace tcs;
 struct tcs_handle {
   tcs_config cfg;
   int sm_count = 148;
-  bool bf16 = false, use_tc = false, fuse_gn = false, fuse_first = true;
+  bool bf16 = false, use_tc = false, fuse_gn = false;
   bool fuse_attn = false;   // the attention block as one tcgen05 kernel (attn_tc.cu); TCS_FUSE_ATTN=0 keeps the four launches
   DevBuf attn_wpack;
   bool fuse_ups = false;    // us1_conv / us2_conv read the half-resolution tensor, the bilinear x2 upsample is blended inside the conv (TCS_FUSE_UPS=0: stand-alone kernel)
@@ -174,7 +174,7 @@ struct tcs_handle {
   ConvTcPlan plan_eps, plan_eps_pair;     // 96 -> 1 output conv on the tensor pipe (N padded to 16)
   DevBuf wpack_out;
   const float* d_bias16 = nullptr;
-  bool tc_out = false, eps_kxn = true;
+  bool eps_kxn = true;
 
   // per-call state
   DevBuf cvec, tvec, tvals, coef, dpm_coef, x, xpred, d0, eps, step_ctr, ycat_tmp, ycont_tmp;
@@ -355,8 +355,6 @@ static int build_plans(tcs_handle* h) {
     return TCS_OK;
   }
   {
-    const char* e = getenv("TCS_TC_OUT");   // 0 = keep the CUDA-core out conv (A/B switch)
-    h->tc_out = !(e && atoi(e) == 0);
     ConvGeom g = geom_of(C_U1B, h->chunk, 1);
     g.ntot = 16;
     g.kx_in_n = h->eps_kxn ? 1 : 0;
@@ -503,12 +501,12 @@ static int forward_chunk(tcs_handle* h, const PassArgs& a, cudaStream_t st, TapR
   { h->launches += 2; TCS_CHECK(launch_gn_apply<T>(raw, 0, part, slots, gnw(key), gnb(key), B, res, res, C, 1, out, h->gnstats.as<float2>(), st)); }
 
   // ---- down1 -------------------------------------------------------------------------------
-  if (h->fuse_first && !(tap && tap->id == 0)) {
+  if (!(tap && tap->id == 0)) {
     ++h->launches;
     TCS_CHECK(launch_first_conv_gn<T>(a.x, h->d_w9, a.tvec, a.tvec_stride, a.step_ptr, a.trow_off, a.cvec, a.ns, a.dup,
                                       gnw("down1.net.1"), gnb("down1.net.1"), h->p64_a.as<T>(), st));
     ++tap_idx;
-  } else {   // unfused variant (also serves the "down1.net.0.raw" debug tap)
+  } else {   // unfused variant: the "down1.net.0.raw" debug tap
     ++h->launches;
     TCS_CHECK(launch_first_conv(a.x, h->d_w9, a.tvec, a.tvec_stride, a.step_ptr, a.trow_off, a.cvec, a.ns, a.dup,
                                 h->raw64.as<float>(), part, st));
@@ -597,7 +595,7 @@ static int forward_chunk(tcs_handle* h, const PassArgs& a, cudaStream_t st, TapR
   CONV_GN(C_U1B, h->raw64.p, 64, 96);
   // ---- out conv + CFG combine ------------------------------------------------------------------
   ++h->launches;
-  if (h->use_tc && h->tc_out) {
+  if (h->use_tc) {
     ConvTcPlan pl = a.dup == 2 ? h->plan_eps_pair : h->plan_eps;
     pl.p.n_mtiles = (a.dup == 2 ? B / 2 : B) * pl.p.tiles_per_img;
     pl.p.guidance = a.guidance;
@@ -938,9 +936,7 @@ int tcs_create(tcs_handle** out, const tcs_config* cfg) {
   h->use_tc = eng == TCS_ENGINE_TCGEN05;
   h->split3 = h->use_tc && !h->bf16;   // fp32 operands as bf16 hi + lo pairs, three MMAs per product (1e-4 parity mode)
   {
-    const char* e = getenv("TCS_FUSE_GN");   // 0 = keep conv -> raw fp32 -> gn_apply (A/B switch)
-    h->fuse_gn = h->use_tc && !h->split3 && cfg->fuse_gn != 0 && !(e && atoi(e) == 0);
-    h->fuse_first = !(e && atoi(e) == 0);
+    h->fuse_gn = h->use_tc && !h->split3 && cfg->fuse_gn != 0;
     const char* eu = getenv("TCS_FUSE_UPS");
     h->fuse_ups = h->use_tc && !h->split3 && !(eu && atoi(eu) == 0);
     const char* ea = getenv("TCS_FUSE_ATTN");
